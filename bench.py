@@ -10,9 +10,14 @@ One sweep = exactly the tutorial loop body (/root/reference/docs/src/tutorials/b
     set_obs! -> recompute_guiding_term!(P only) -> find_W_for_X! + loglikhd! + draw_proposal_path! -> accept_reject_proposal_path!
     -> (N > 1: all-reduce of ll sums / accept counts)
 and advances every chain by S = 20,000 guided Euler-Maruyama steps.  One timed "step" = R consecutive sweeps (R stated in `config`,
-chosen after the warm-up so that the K timed steps last >= 2.5 s: long enough for the clock sampler); units per step = R x M x S.
+chosen after the warm-up so that the K timed steps last >= 2.5 s: long enough for the clock sampler; with --dump-outputs, a fixed number
+of sweeps per config instead, so that the dumped state does not depend on a measured time); units per step = R x M x S.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3|c2|c4|c5] [--chains M_per_gpu] [--impl reference]
+                    [--dump-outputs DIR]
+
+After build(), bench.py writes nothing into the tree it runs from (which may be read-only): what it compiles goes to a temporary
+directory.
 """
 import argparse
 import json
@@ -20,6 +25,7 @@ import math
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -27,6 +33,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # no __pycache__ in the tree for the modules only the benchmark imports
 
 METRIC = "guided path updates/sec (chains x EM steps/s, FP64)"
 UNIT = "guided EM steps/s"
@@ -35,6 +42,13 @@ ALGO_BYTES = {  # SURVEY.md §8(d): per chain per EM step of draw_proposal_path!
     "c2": (48, 88), "c3": (72, 144), "c4": (96, 208), "c5": (64, 280), "c1": (32, 72),
 }
 MIN_TIMED_S = 2.5
+# --dump-outputs: the dumped state depends on how many sweeps ran, so the timed region holds a fixed number of sweeps per config (the same
+# on every rank) instead of one sized from a measured time: about MIN_TIMED_S of sweeps of the config's ensemble on one B200 at the
+# sweep times measured in profiles/r02v_bench_c1.json, r02v_bench_c2.json, r02aw_bench_default.json, r02x_bench_c4.json and
+# r02ae_bench_c5.json (0.31 / 1.54 / 3.44 / 16.3 / 225 ms; SM clock 1965 MHz, power limit not recorded)
+DUMP_TIMED_SWEEPS = {"c1": 8000, "c2": 1600, "c3": 720, "c4": 150, "c5": 11}
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE_CHAINS = 32
 
 
 def parse():
@@ -59,7 +73,15 @@ def parse():
     ap.add_argument("--sweep-mode", type=int, default=0, help="fused pass: 0 auto, 1 register-tile kernel, 2 software-pipelined, 3 / 4 warp-specialised (wide / compact), 5 step-parallel (4 lanes per (chain, block))")
     ap.add_argument("--fwd-lanes", type=int, default=0, help="lanes per (chain, block) in the forward kernel (0: automatic)")
     ap.add_argument("--eager-noise", action="store_true", help="the sweep stores W_acc / W° (default: lazy noise, rebuilt from X on demand)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy: stats, ll, ll_proposal, "
+                         "accepted [n_blocks, M], and X, X_proposal [NP, d, n] of n <= %d chains drawn by np.random.default_rng(0); at "
+                         "most %d MB.  Unless --sweeps-per-step is given, R is then a fixed number of sweeps per config so that runs "
+                         "with the same arguments run the same sweeps" % (DUMP_SAMPLE_CHAINS, DUMP_MAX_BYTES >> 20))
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
+    return a
 
 
 def workload_config(cfg, M_total, prob):
@@ -75,20 +97,15 @@ def workload_config(cfg, M_total, prob):
 
 # ------------------------------------------------------------------------------------------------ CPU arm (oracle port)
 def native_oracle():
-    """the OpenMP flavour of the oracle rebuilt for THIS host (-O3 -march=native) when gcc is present; else the shipped generic build"""
+    """the OpenMP flavour of the oracle rebuilt for THIS host (-O3 -march=native) in a temporary directory when gcc is present; else the
+    shipped generic build"""
     from oracle import orc
     src = os.path.join(ROOT, "oracle", "dmt_oracle.c")
     try:
-        import hashlib
-        flags = [ln for ln in open("/proc/cpuinfo") if ln.startswith(("flags", "model name"))][:2]
-        tag = hashlib.sha1("".join(flags).encode()).hexdigest()[:10]   # a binary built for another host's CPU must not be reused
-    except Exception:
-        tag = "host"
-    out = os.path.join(ROOT, "oracle", "libdmt_oracle_omp_native_%s.so" % tag)
-    try:
-        if not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(src):
+        with tempfile.TemporaryDirectory() as tmp:   # the loaded library stays mapped after its file is removed
+            out = os.path.join(tmp, "libdmt_oracle_omp_native.so")
             subprocess.run(["gcc", "-std=c99", "-O3", "-march=native", "-fopenmp", "-fPIC", "-shared", "-o", out, src, "-lm"], check=True, capture_output=True)
-        return orc.load(path=out), "-O3 -march=native -fopenmp"
+            return orc.load(path=out), "-O3 -march=native -fopenmp"
     except Exception:
         return orc.load(omp=True), "-O3 -fopenmp (generic x86-64)"
 
@@ -395,6 +412,24 @@ def self_check(run, it):
     return out
 
 
+def dump_last_step(run, l, stats, out_dir):
+    """what the last timed sweep (layout l) left for its caller: the all-reduced stats, per-(block, chain) ll / ll° and decisions,
+    and the accepted / proposed paths of a fixed sample of chains"""
+    ctx, prob = run.ctx, run.prob
+    out = {"stats": np.asarray(stats, dtype=np.float64), "ll": ctx.get_ll(l, 0), "ll_proposal": ctx.get_ll(l, 1),
+           "accepted": ctx.get_last_accept(l).astype(np.float32)}
+    fixed = sum(v.nbytes for v in out.values())
+    per_chain = 2 * 8 * ctx.NP * prob.d
+    n = min(prob.M, DUMP_SAMPLE_CHAINS, max(0, (DUMP_MAX_BYTES - fixed) // per_chain))
+    if n == 0:
+        raise ValueError("--dump-outputs: the per-chain outputs of %d chains exceed %d MB" % (prob.M, DUMP_MAX_BYTES >> 20))
+    chains = np.sort(np.random.default_rng(0).choice(prob.M, n, replace=False))
+    out["X"], out["X_proposal"] = ctx.get_X_chains(chains, 0), ctx.get_X_chains(chains, 1)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 def gpu_arm(a):
     import torch
     import torch.distributed as dist
@@ -425,7 +460,9 @@ def gpu_arm(a):
     for _ in range(max(a.warmup, 3)):   # warm-up steps (cover the guiding-cache build on both layouts)
         for _ in range(max(R, run.nlay)):
             run.sweep(it, False); it += 1
-    if a.sweeps_per_step <= 0:          # estimate the sweep time, then fix R for the timed region
+    if a.sweeps_per_step <= 0 and a.dump_outputs:
+        R = max(1, int(math.ceil(DUMP_TIMED_SWEEPS[a.config] / a.steps)))
+    elif a.sweeps_per_step <= 0:        # estimate the sweep time, then fix R for the timed region
         ms_est, _, _, it = run.timed_run(it, 1, 2 * run.nlay, timed_kernels=False)
         per_sweep = ms_est / (2 * run.nlay) * 1e-3
         R = int(run.max_over_ranks(max(1, int(math.ceil(MIN_TIMED_S / (a.steps * per_sweep))))))
@@ -435,6 +472,8 @@ def gpu_arm(a):
     t_wall1 = time.time()
     launches = _lib.launch_count() - n0
     clocks = sampler.stop(t_wall0, t_wall1)
+    if a.dump_outputs and rank == 0:
+        dump_last_step(run, (it - 1) % run.nlay, last, a.dump_outputs)
     units_per_step = R * M_job * prob.steps_per_chain
     value = units_per_step * a.steps / (ms_total * 1e-3)
     ms_per_sweep = ms_total / (a.steps * R)
