@@ -473,7 +473,7 @@ class Ctx:
         self._ck(self.lib.dmt_set_fwd_lanes(self.h, int(lanes)))
 
     def set_sweep_mode(self, mode):
-        """fused blocking-sweep pass: 0 = automatic, 1 = register-tile kernel, 2 = software-pipelined kernel, 3 / 4 = warp-specialised kernel, wide / compact shape, 5 = step-parallel kernel (or error)"""
+        """fused blocking-sweep pass: 0 = automatic, 1 = register-tile kernel, 2 = software-pipelined kernel, 3 = warp-specialised kernel, 5 = step-parallel kernel (or error)"""
         self._ck(self.lib.dmt_set_sweep_mode(self.h, int(mode)))
 
     def last_forward_kernel(self):

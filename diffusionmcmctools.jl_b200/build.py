@@ -1,7 +1,7 @@
 """Build libdmt.so (hand-written sm_100a CUDA + C ABI) in-tree with nvcc.  No GPU needed to compile.
 
     python build.py [--force] [-v]                     -> libdmt.so
-    python build.py --tag pf0 -DDMT_PF_DIST=0 ...      -> libdmt_pf0.so   (tuning variants; select with DMT_LIB=<path>)
+    python build.py --tag tpb32 -DDMT_FWD_TPB=32 ...   -> libdmt_tpb32.so (tuning variants; select with DMT_LIB=<path>)
 """
 import os
 import subprocess

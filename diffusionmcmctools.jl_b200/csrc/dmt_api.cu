@@ -9,14 +9,15 @@
 #include "tsit5_kernel.cuh"
 
 #include <algorithm>
+#include <atomic>
 #include <nvtx3/nvToolsExt.h> // header-only: ranges are emitted when DMT_NVTX=1 and a profiler is attached
-#include <type_traits>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <dlfcn.h>
 #include <stdexcept>
 #include <string>
+#include <unordered_map>
 #include <vector>
 
 using namespace dmt;
@@ -47,7 +48,7 @@ struct DmtError : std::runtime_error {
     } while (0)
 
 std::string g_create_error;
-unsigned long long g_launches = 0; // kernels launched by this library in this process (dmt_launch_count; a ctx is single-threaded)
+std::atomic<unsigned long long> g_launches{0}; // kernels launched by this library in this process, all contexts (dmt_launch_count)
 
 struct ModelDims { int D, DW, NPAR; bool constdiff; };
 bool model_dims(int model, ModelDims &md) {
@@ -176,9 +177,10 @@ struct dmt_ctx {
     cudaEvent_t ev_gathered = nullptr, ev_copied = nullptr, ev_hist = nullptr;
     DevBuf<double> d_snap;
     DevBuf<int> d_snap_sel;
-    bool tma_ok = false;     // P == M with the identity pset map: the TMA fast path of fwd_kernel is usable
     bool pipe_ok = false;    // P == M with the identity pset map: a warp's guiding-term sectors are contiguous (sweep_pipe_kernel)
-    int sweep_mode = 0;      // dmt_set_sweep_mode: 0 = automatic (pipelined where eligible), 1 = register-tile kernel, 2 = pipelined or error
+    int sweep_mode = 0;      // dmt_set_sweep_mode: 0 = automatic (pick_sweep), 1 = register-tile kernel, 2 / 3 / 5 = pipelined /
+                             // warp-specialised / step-parallel kernel or error
+    std::unordered_map<const void *, size_t> resident; // kernel -> CTAs resident at once on this context's device (resident_ctas)
     bool lazy_W = false;     // dmt_set_lazy_noise: blocking sweeps do not materialise W_acc / W°
     char last_fwd_kernel[96] = ""; // name and mapping of the forward kernel launched last (dmt_get_last_forward_kernel)
     int W_stale_layout = -1; // >= 0: W_acc is not materialised; K5 over this layout rebuilds it (ensure_W)
@@ -212,70 +214,59 @@ void check_range(dmt_ctx *c, int k0, int k1) { REQUIRE(0 <= k0 && k0 <= k1 && k1
 dim3 chain_grid(dmt_ctx *c, int ny, int tpb) { return dim3((c->M + tpb - 1) / tpb, ny, 1); }
 dim3 pset_grid(dmt_ctx *c, int ny, int tpb, int nz = 1) { return dim3((c->P + tpb - 1) / tpb, ny, nz); }
 
-template <class MD, int OP, bool TMA, int G> void launch_fwd_lanes(dmt_ctx *c, Layout &L, const FwdArgs &fa, int *wave_threads) {
-    constexpr int TPB = (MD::D >= 6) ? 32 : FWD_TPB; // wide guiding terms: smaller CTAs
-    constexpr size_t smem = fwd_smem_bytes<MD, TPB, TMA>();
-    static bool attr_done[64] = {};
-    static int wave[64] = {};
-    const int dev = c->cfg.device & 63;
-    if (!attr_done[dev]) {
-        CK(cudaFuncSetAttribute(fwd_kernel<MD, OP, TPB, TMA, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int per_sm = 0, sms = 0;
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fwd_kernel<MD, OP, TPB, TMA, G>, TPB, smem));
-        CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
-        wave[dev] = per_sm * sms * TPB; // threads resident at once
-        attr_done[dev] = true;
-    }
-    if (wave_threads) { *wave_threads = wave[dev]; return; } // query only
+// CTAs of `kernel` resident at once on the context's device with `threads` threads and `smem` bytes of dynamic shared memory each.
+// Raises the kernel's dynamic-shared-memory limit to `smem` first, so every launch of the kernels below goes through here once
+// before its first launch.  Cached per context: the answer depends on the device, and a context owns one device.
+template <class Kernel> size_t resident_ctas(dmt_ctx *c, Kernel *kernel, int threads, size_t smem) {
+    const auto it = c->resident.find((const void *)kernel);
+    if (it != c->resident.end()) return it->second;
+    int per_sm = 0, sms = 0;
+    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
+    return c->resident[(const void *)kernel] = (size_t)per_sm * sms;
+}
+
+// ---- the register-tile kernel (fwd_kernel.cuh): G lanes per (chain, block), G > 1 for the ops that draw normals
+template <int OP> constexpr bool fwd_coop() { return OP == OP_DRAW || OP == OP_INIT || OP == OP_SWEEP; }
+template <class MD> constexpr int fwd_tpb() { return MD::D >= 6 ? 32 : FWD_TPB; } // wide guiding terms: smaller CTAs
+template <class MD, int OP, int G> size_t fwd_wave_threads(dmt_ctx *c) {
+    return resident_ctas(c, fwd_kernel<MD, OP, fwd_tpb<MD>(), G>, fwd_tpb<MD>(), 0) * fwd_tpb<MD>();
+}
+template <class MD, int OP, int G> void launch_fwd_g(dmt_ctx *c, Layout &L, const FwdArgs &fa) {
+    constexpr int TPB = fwd_tpb<MD>();
+    fwd_wave_threads<MD, OP, G>(c);
     const dim3 grid((unsigned)(((size_t)c->M * G + TPB - 1) / TPB), L.nb, 1);
-    snprintf(c->last_fwd_kernel, sizeof(c->last_fwd_kernel), "fwd_kernel<op=%d, lanes=%d%s%s>", OP, G, TMA ? ", tma" : "", (OP == OP_SWEEP && fa.lazy_w) ? ", lazy" : "");
-    ++g_launches, fwd_kernel<MD, OP, TPB, TMA, G><<<grid, TPB, smem, c->stream>>>(c->dev, L.dev, fa);
+    snprintf(c->last_fwd_kernel, sizeof(c->last_fwd_kernel), "fwd_kernel<op=%d, lanes=%d%s>", OP, G, (OP == OP_SWEEP && fa.lazy_w) ? ", lazy" : "");
+    ++g_launches, fwd_kernel<MD, OP, TPB, G><<<grid, TPB, 0, c->stream>>>(c->dev, L.dev, fa);
 }
-// Lanes per (chain, block): 1 when the ensemble fills the GPU by itself; 2, 4 or 8 when M x blocks x lanes still fits one wave
-// of the cooperative instantiation (the generator is split over the lanes, fwd_kernel.cuh).  DMT_FWD_LANES overrides.
-template <class MD, int OP, bool TMA> void launch_fwd_variant(dmt_ctx *c, Layout &L, const FwdArgs &fa) {
-    constexpr bool COOP_OK = !TMA && (OP == OP_DRAW || OP == OP_INIT || OP == OP_SWEEP);
-    int lanes = 1;
-    if (COOP_OK) {
-        static int env_forced = -1;
-        if (env_forced < 0) { const char *e = getenv("DMT_FWD_LANES"); env_forced = e ? atoi(e) : 0; }
-        const int forced = c->fwd_lanes ? c->fwd_lanes : env_forced;
-        const size_t units = (size_t)c->M * L.nb;
-        int w = 0;
-        if (forced) lanes = forced;
-        else if (MD::DW >= 2 && OP == OP_SWEEP) {
-            // the fused sweep: two lanes whenever the doubled grid still fits one wave — measured best at every ensemble size where
-            // it applies (Lorenz, lazy noise, fused pass in ms for 512 / 768 / 1024 / 1536 chains: 1 lane 2.12 / 2.14 / 2.15 / 2.17,
-            // 2 lanes 1.03 / 1.05 / 1.35 / 1.39, 4 lanes 1.14 / 1.17 / 1.81 / 2.29; profiles/r02_tuning.md)
-            launch_fwd_lanes<MD, OP, false, 2>(c, L, fa, &w);
-            if (units * 2 <= (size_t)w) lanes = 2;
-        } else if (MD::DW >= 2) { // with one Wiener coordinate the generator is a small part of the tile: redundant lanes only cost issue slots
-                                 // (Jansen-Rit draw, 8192 chains: 87 ms with 1 lane, 121 ms with 4)
-            launch_fwd_lanes<MD, OP, false, 8>(c, L, fa, &w);
-            if (units * 8 <= (size_t)w) lanes = 8;
-            else {
-                launch_fwd_lanes<MD, OP, false, 4>(c, L, fa, &w);
-                if (units * 4 <= (size_t)w) lanes = 4;
-                else {
-                    launch_fwd_lanes<MD, OP, false, 2>(c, L, fa, &w);
-                    if (units * 2 <= (size_t)w) lanes = 2;
-                }
-            }
-        }
+template <class MD, int OP> void launch_fwd_tile(dmt_ctx *c, Layout &L, const FwdArgs &fa, int lanes) {
+    if constexpr (fwd_coop<OP>()) {
+        if (lanes == 8) return launch_fwd_g<MD, OP, 8>(c, L, fa);
+        if (lanes == 4) return launch_fwd_g<MD, OP, 4>(c, L, fa);
+        if (lanes == 2) return launch_fwd_g<MD, OP, 2>(c, L, fa);
     }
-    if (COOP_OK && lanes == 8) launch_fwd_lanes<MD, OP, false, COOP_OK ? 8 : 1>(c, L, fa, nullptr);
-    else if (COOP_OK && lanes == 4) launch_fwd_lanes<MD, OP, false, COOP_OK ? 4 : 1>(c, L, fa, nullptr);
-    else if (COOP_OK && lanes == 2) launch_fwd_lanes<MD, OP, false, COOP_OK ? 2 : 1>(c, L, fa, nullptr);
-    else launch_fwd_lanes<MD, OP, TMA, 1>(c, L, fa, nullptr);
+    launch_fwd_g<MD, OP, 1>(c, L, fa);
 }
-template <class MD, int OP> void launch_fwd_model(dmt_ctx *c, Layout &L, const FwdArgs &fa) {
-#ifdef DMT_WITH_TMA
-    // TMA path (opt-in build, -DDMT_WITH_TMA, and DMT_TMA=1 at run time): every chain owns its pset in chain order and the law
-    // parity is uniform, so a warp's H,F chunk is contiguous.  Measured SLOWER than the LDG.256 path inside the real kernel
-    // (3.83 vs 3.29 ms, profiles/r01_tuning.md) although faster on the bare memory pattern — kept for the next round's work.
-    if (c->tma_ok && !c->parP_mixed) { launch_fwd_variant<MD, OP, true>(c, L, fa); return; }
-#endif
-    launch_fwd_variant<MD, OP, false>(c, L, fa);
+// Lanes per (chain, block): dmt_set_fwd_lanes if set; else 1 when the ensemble fills the GPU by itself, and 2, 4 or 8 when
+// chains x blocks x lanes still fits one wave (the generator is split over the lanes, fwd_kernel.cuh).
+template <class MD, int OP> int tile_lanes(dmt_ctx *c, const Layout &L) {
+    if constexpr (fwd_coop<OP>()) {
+        if (c->fwd_lanes) return c->fwd_lanes;
+        // with one Wiener coordinate the generator is a small part of the tile: redundant lanes only cost issue slots
+        // (Jansen-Rit draw, 8192 chains: 87 ms with 1 lane, 121 ms with 4)
+        if (MD::DW < 2) return 1;
+        const size_t units = (size_t)c->M * L.nb;
+        if (OP != OP_SWEEP) {
+            if (units * 8 <= fwd_wave_threads<MD, OP, 8>(c)) return 8;
+            if (units * 4 <= fwd_wave_threads<MD, OP, 4>(c)) return 4;
+        }
+        // the fused sweep: two lanes whenever the doubled grid still fits one wave — measured best at every ensemble size where
+        // it applies (Lorenz, lazy noise, fused pass in ms for 512 / 768 / 1024 / 1536 chains: 1 lane 2.12 / 2.14 / 2.15 / 2.17,
+        // 2 lanes 1.03 / 1.05 / 1.35 / 1.39, 4 lanes 1.14 / 1.17 / 1.81 / 2.29; profiles/r02_tuning.md)
+        if (units * 2 <= fwd_wave_threads<MD, OP, 2>(c)) return 2;
+    }
+    return 1;
 }
 
 void ensure_guiding(dmt_ctx *c, Layout &L);
@@ -287,163 +278,91 @@ bool covers_all_intervals(dmt_ctx *c, const Layout &L) {
     return std::all_of(seen.begin(), seen.end(), [](char s) { return s != 0; });
 }
 
-// wave_warps != nullptr: only report how many warps of this instantiation are resident at once on the device
-template <class MD, int G> void launch_sweep_pipe_g(dmt_ctx *c, Layout &L, const FwdArgs &fa, bool lazy, size_t *wave_warps = nullptr) {
+// ---- the other kernels of the fused sweep pass.  All three need one parameter set per chain in chain order, uniform law parity
+// and device RNG; each is compiled with and without lazy noise.
+// the software-pipelined sweep (sweep_kernel.cuh): one lane per (chain, block), guiding term through a TMA shared-memory ring
+template <class MD, bool LAZY> void launch_sweep_pipe(dmt_ctx *c, Layout &L, const FwdArgs &fa) {
     constexpr size_t smem = sweep_pipe_smem<MD>();
-    static bool attr_done[64][2] = {};
-    static size_t wave[64][2] = {};
-    const int dev = c->cfg.device & 63;
-    if (!attr_done[dev][lazy]) {
-        int per_sm = 0, sms = 0;
-        if (lazy) {
-            CK(cudaFuncSetAttribute(sweep_pipe_kernel<MD, true, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sweep_pipe_kernel<MD, true, G>, 32, smem));
-        } else {
-            CK(cudaFuncSetAttribute(sweep_pipe_kernel<MD, false, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sweep_pipe_kernel<MD, false, G>, 32, smem));
-        }
-        CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
-        wave[dev][lazy] = (size_t)per_sm * sms;
-        attr_done[dev][lazy] = true;
-    }
-    if (wave_warps) { *wave_warps = wave[dev][lazy]; return; }
-    const dim3 grid((unsigned)((c->M + 32 / G - 1) / (32 / G)), L.nb, 1);
-    snprintf(c->last_fwd_kernel, sizeof(c->last_fwd_kernel), "sweep_pipe_kernel<lanes=%d%s>", G, lazy ? ", lazy" : "");
-    if (lazy) ++g_launches, sweep_pipe_kernel<MD, true, G><<<grid, 32, smem, c->stream>>>(c->dev, L.dev, fa);
-    else ++g_launches, sweep_pipe_kernel<MD, false, G><<<grid, 32, smem, c->stream>>>(c->dev, L.dev, fa);
-}
-// the warp-specialised sweep (sweep_ws_kernel.cuh): a pipeline of warps per group of 32 chains and block.  Two shapes: WsSmall for
-// ensembles that cannot fill the GPU (more helper warps around the one recursion warp, deep rings), WsLarge for full ones
-#ifndef DMT_SP_MAX_UNITS_DEFAULT
-#define DMT_SP_MAX_UNITS_DEFAULT 14080 // 1280 chains x 11 blocks (12 resident warps per SM at 168 registers).  Measured (Lorenz, lazy noise, fused
-                                       // pass in ms at 512 / 1024 / 1280 chains x 10 blocks; profiles/r02_tuning.md §4e): step-parallel 0.83 / 1.10 /
-                                       // 1.18, two lanes per (chain, block) in the register-tile kernel 1.03 / 1.35 / 1.37
-#endif
-#ifndef DMT_WS_NR // (tuning builds: -DDMT_WS_NR=.. -DDMT_WS_NSG=.. -DDMT_WS_NSR=..)
-#define DMT_WS_NR 6
-#endif
-#ifndef DMT_WS_NSG
-#define DMT_WS_NSG 8
-#endif
-#ifndef DMT_WS_NSR // depth of the Z, D and X rings
-#define DMT_WS_NSR 4
-#endif
-// ring depths by state dimension: a stage of the G ring is (d(d+1)/2 + d) KiB, the D ring holds the same again per slot
-template <class MD> struct WsShapeOf { using type = WsShape<DMT_WS_NR, (MD::D <= 3 ? DMT_WS_NSG : MD::D == 4 ? 6 : 3), (MD::D <= 3 ? DMT_WS_NSR : MD::D == 4 ? 3 : 2)>; };
-// the compact shape (two CTAs per SM: at most ~113 KB of shared memory each); the wide states do not fit twice
-#ifndef DMT_WSC_NSG
-#define DMT_WSC_NSG 6
-#endif
-#ifndef DMT_WSC_NSR
-#define DMT_WSC_NSR 2
-#endif
-template <class MD> struct WsCompactOf { using type = WsShape<2, (MD::D <= 3 ? DMT_WSC_NSG : 4), DMT_WSC_NSR, true>; };
-template <class MD> constexpr bool ws_compact_fits() { return sweep_ws_smem<MD, typename WsCompactOf<MD>::type>() <= 113 * 1024; }
-template <class MD, class SH, int MINB> void launch_sweep_ws(dmt_ctx *c, Layout &L, const FwdArgs &fa, bool lazy, size_t *wave_ctas = nullptr) {
-    constexpr size_t smem = sweep_ws_smem<MD, SH>();
-    static_assert(smem <= 227 * 1024, "the rings of the warp-specialised sweep must fit one SM's shared memory");
-    static bool attr_done[64][2] = {};
-    static size_t wave[64][2] = {};
-    const int dev = c->cfg.device & 63;
-    if (!attr_done[dev][lazy]) {
-        int per_sm = 0, sms = 0;
-        if (lazy) {
-            CK(cudaFuncSetAttribute(sweep_ws_kernel<MD, true, SH, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sweep_ws_kernel<MD, true, SH, MINB>, SH::THREADS, smem));
-        } else {
-            CK(cudaFuncSetAttribute(sweep_ws_kernel<MD, false, SH, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sweep_ws_kernel<MD, false, SH, MINB>, SH::THREADS, smem));
-        }
-        CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
-        wave[dev][lazy] = (size_t)per_sm * sms;
-        attr_done[dev][lazy] = true;
-    }
-    if (wave_ctas) { *wave_ctas = wave[dev][lazy]; return; }
+    resident_ctas(c, sweep_pipe_kernel<MD, LAZY>, 32, smem);
     const dim3 grid((unsigned)((c->M + 31) / 32), L.nb, 1);
-    snprintf(c->last_fwd_kernel, sizeof(c->last_fwd_kernel), "sweep_ws_kernel<%s, %s>", SH::COMPACT ? "compact" : "wide", lazy ? "lazy" : "eager");
-    if (lazy) ++g_launches, sweep_ws_kernel<MD, true, SH, MINB><<<grid, SH::THREADS, smem, c->stream>>>(c->dev, L.dev, fa);
-    else ++g_launches, sweep_ws_kernel<MD, false, SH, MINB><<<grid, SH::THREADS, smem, c->stream>>>(c->dev, L.dev, fa);
+    snprintf(c->last_fwd_kernel, sizeof(c->last_fwd_kernel), "sweep_pipe_kernel<lanes=1%s>", LAZY ? ", lazy" : "");
+    ++g_launches, sweep_pipe_kernel<MD, LAZY><<<grid, 32, smem, c->stream>>>(c->dev, L.dev, fa);
+}
+// the warp-specialised sweep (sweep_ws_kernel.cuh): a pipeline of 16 warps per group of 32 chains and block, one CTA per SM.  Six
+// generator warps; ring depths by state dimension (a stage of the G ring is (d(d+1)/2 + d) KiB, the D ring holds the same again per
+// slot): G ring 8 / 6 / 3 stages and Z, D, X rings 4 / 3 / 2 slots for d <= 3 / d = 4 / d >= 5
+template <class MD> using WsWide = WsShape<6, (MD::D <= 3 ? 8 : MD::D == 4 ? 6 : 3), (MD::D <= 3 ? 4 : MD::D == 4 ? 3 : 2)>;
+template <class MD, bool LAZY> size_t ws_resident_ctas(dmt_ctx *c) {
+    constexpr size_t smem = sweep_ws_smem<MD, WsWide<MD>>();
+    static_assert(smem <= 227 * 1024, "the rings of the warp-specialised sweep must fit one SM's shared memory");
+    return resident_ctas(c, sweep_ws_kernel<MD, LAZY, WsWide<MD>>, WsWide<MD>::THREADS, smem);
+}
+template <class MD, bool LAZY> void launch_sweep_ws(dmt_ctx *c, Layout &L, const FwdArgs &fa) {
+    using SH = WsWide<MD>;
+    ws_resident_ctas<MD, LAZY>(c);
+    const dim3 grid((unsigned)((c->M + 31) / 32), L.nb, 1);
+    snprintf(c->last_fwd_kernel, sizeof(c->last_fwd_kernel), "sweep_ws_kernel<wide, %s>", LAZY ? "lazy" : "eager");
+    ++g_launches, sweep_ws_kernel<MD, LAZY, SH><<<grid, SH::THREADS, sweep_ws_smem<MD, SH>(), c->stream>>>(c->dev, L.dev, fa);
 }
 // the step-parallel sweep (sweep_sp_kernel.cuh): four lanes per (chain, block), lane = step of the tile
-template <class MD> void launch_sweep_sp(dmt_ctx *c, Layout &L, const FwdArgs &fa, bool lazy) {
+template <class MD, bool LAZY> void launch_sweep_sp(dmt_ctx *c, Layout &L, const FwdArgs &fa) {
     const dim3 grid((unsigned)((c->M + 7) / 8), L.nb, 1);
-    snprintf(c->last_fwd_kernel, sizeof(c->last_fwd_kernel), "sweep_sp_kernel<step lanes=4%s>", lazy ? ", lazy" : "");
-    if (lazy) ++g_launches, sweep_sp_kernel<MD, true><<<grid, 32, 0, c->stream>>>(c->dev, L.dev, fa);
-    else ++g_launches, sweep_sp_kernel<MD, false><<<grid, 32, 0, c->stream>>>(c->dev, L.dev, fa);
-}
-// the software-pipelined sweep (sweep_kernel.cuh): one parameter set per chain in chain order, uniform law parity, device RNG
-template <class MD> bool launch_sweep_pipe(dmt_ctx *c, Layout &L, const FwdArgs &fa) {
-    static int env_off = -1;
-    if (env_off < 0) env_off = getenv("DMT_NO_SWEEP_PIPE") ? 1 : 0;
-    const bool eligible = c->pipe_ok && !c->parP_mixed && !fa.Z && fa.skip == 0;
-    if (c->sweep_mode >= 2 && !eligible)
-        throw DmtError(DMT_ERR_UNSUPPORTED, "pipelined sweep needs one parameter set per chain in chain order, uniform law parity and device RNG");
-    if (!eligible || c->sweep_mode == 1 || (c->sweep_mode == 0 && (c->fwd_lanes != 0 || env_off))) return false;
-    const bool lazy = c->lazy_W && covers_all_intervals(c, L);
-    {   // the warp-specialised kernel: forced by modes 3 (wide shape, one CTA per SM) and 4 (compact shape, two per SM); automatic while its
-        // grid fits ONE round of the wide shape, else one round of the compact one (profiles/r02_tuning.md: a round costs ~0.5 ms on C3
-        // whatever the ensemble size, so a second round loses to the one-thread-per-(chain, block) kernels)
-        using Wide = typename WsShapeOf<MD>::type;
-        using Compact = typename WsCompactOf<MD>::type;
-        constexpr bool CFITS = ws_compact_fits<MD>();
-        using CompactOrWide = typename std::conditional<CFITS, Compact, Wide>::type; // (never launched when it does not fit)
-        const size_t units = (size_t)((c->M + 31) / 32) * L.nb;
-        size_t wave_w = 0, wave_c = 0;
-        launch_sweep_ws<MD, Wide, 1>(c, L, fa, lazy, &wave_w);
-        (void)wave_c;
-        static int ws_rounds = -1;
-        if (ws_rounds < 0) { const char *e = getenv("DMT_WS_MAX_ROUNDS"); ws_rounds = e ? atoi(e) : 1; }
-        const bool automatic = c->sweep_mode == 0 && c->fwd_lanes == 0;
-        static int sp_max_units = -1; // automatic: the step-parallel kernel while (chain, block) units <= this (0: never)
-        if (sp_max_units < 0) { const char *e = getenv("DMT_SP_MAX_UNITS"); sp_max_units = e ? atoi(e) : DMT_SP_MAX_UNITS_DEFAULT; }
-        if (c->sweep_mode == 5 || (automatic && MD::DW >= 2 && !(wave_w > 0 && units <= (size_t)ws_rounds * wave_w) && (size_t)c->M * L.nb <= (size_t)sp_max_units)) {
-            launch_sweep_sp<MD>(c, L, fa, lazy);
-            if (lazy) c->W_stale_layout = L.dev.id;
-            return true;
-        }
-        if (c->sweep_mode == 4 && !CFITS) throw DmtError(DMT_ERR_UNSUPPORTED, "the compact warp-specialised sweep does not fit this model's state dimension");
-        if (c->sweep_mode == 3 || (automatic && wave_w > 0 && units <= (size_t)ws_rounds * wave_w)) {
-            launch_sweep_ws<MD, Wide, 1>(c, L, fa, lazy);
-            if (lazy) c->W_stale_layout = L.dev.id;
-            return true;
-        }
-        // (the compact shape is never chosen automatically: one round of it costs 1.03 ms on C3, the same as two lanes per (chain, block)
-        // in the register-tile kernel — 512 / 768 / 896 chains: 1.03 / 1.04 / 1.04 against 1.03 / 1.05 / — ms)
-        if (CFITS && c->sweep_mode == 4) {
-            launch_sweep_ws<MD, CompactOrWide, CFITS ? 2 : 1>(c, L, fa, lazy);
-            if (lazy) c->W_stale_layout = L.dev.id;
-            return true;
-        }
-    }
-    // automatic choice: with the noise stored every sweep the pipelined kernel's live set (two more tile buffers) spills and it loses to the
-    // register-tile kernel (3.9 against 3.5 ms on C3, profiles/r02_tuning.md); it wins where the noise is lazy (2.44 against 3.5 ms)
-    if (c->sweep_mode == 0 && !lazy) return false;
-    // lanes per (chain, block) in the pipelined kernel: one.  (The 4-lane instantiation exists and can be forced with dmt_set_fwd_lanes(4), but
-    // it never won: 2.56 against 1.40 ms at 1024 chains.)  Mid-size ensembles — a doubled grid of the register-tile kernel still fits one
-    // wave — go to that kernel with two lanes per (chain, block), which splits the generator: 1.35 against 1.40 ms at 1024 chains, 1.03
-    // against 1.38 ms at 512 (profiles/r02_tuning.md).
-    constexpr int GW = MD::DW >= 2 ? 4 : 1; // the wide mappings exist for these models only
-    constexpr int G2 = MD::DW >= 2 ? 2 : 1;
-    bool g4 = false, g2 = false;
-    if (c->fwd_lanes != 0) { // dmt_set_fwd_lanes together with dmt_set_sweep_mode(2): force the mapping
-        if (c->fwd_lanes != 1 && !((c->fwd_lanes == 4 || c->fwd_lanes == 2) && GW == 4))
-            throw DmtError(DMT_ERR_UNSUPPORTED, "the pipelined sweep maps 1 or (models with >= 2 Wiener coordinates) 2 or 4 lanes to a (chain, block)");
-        g4 = c->fwd_lanes == 4;
-        g2 = c->fwd_lanes == 2;
-    } else if (c->sweep_mode == 0 && MD::DW >= 2) {
-        int w2 = 0;
-        launch_fwd_lanes<MD, OP_SWEEP, false, 2>(c, L, fa, &w2);
-        if ((size_t)c->M * L.nb * 2 <= (size_t)w2) return false;
-    }
-    if (g2) launch_sweep_pipe_g<MD, G2>(c, L, fa, lazy);
-    else if (g4) launch_sweep_pipe_g<MD, GW>(c, L, fa, lazy);
-    else launch_sweep_pipe_g<MD, 1>(c, L, fa, lazy);
-    if (lazy) c->W_stale_layout = L.dev.id;
-    return true;
+    snprintf(c->last_fwd_kernel, sizeof(c->last_fwd_kernel), "sweep_sp_kernel<step lanes=4%s>", LAZY ? ", lazy" : "");
+    ++g_launches, sweep_sp_kernel<MD, LAZY><<<grid, 32, 0, c->stream>>>(c->dev, L.dev, fa);
 }
 
-template <int OP> void launch_fwd(dmt_ctx *c, Layout &L, const FwdArgs &fa_in) {
-    FwdArgs fa = fa_in;
+// What the fused sweep pass (K5 + K4 + K3 + K2 + K4, OP_SWEEP) launches: the kernel, the register-tile kernel's lanes per
+// (chain, block), and whether the pass skips the W_acc / W° stores (dmt_set_lazy_noise; then W is rebuilt on demand, ensure_W)
+struct SweepChoice {
+    enum Kernel { TILE, PIPE, WS, SP } kernel;
+    int lanes;
+    bool lazy;
+};
+template <class MD> SweepChoice pick_sweep(dmt_ctx *c, const Layout &L, const FwdArgs &fa) {
+    const bool lazy = c->lazy_W && !fa.Z && covers_all_intervals(c, L);
+    const bool eligible = c->pipe_ok && !c->parP_mixed && !fa.Z && fa.skip == 0;
+    const int mode = c->sweep_mode;
+    if (mode >= 2) { // forced: 2 pipelined, 3 warp-specialised, 5 step-parallel
+        REQUIRE(eligible, DMT_ERR_UNSUPPORTED, "pipelined sweep needs one parameter set per chain in chain order, uniform law parity and device RNG");
+        if (mode == 3) return {SweepChoice::WS, 1, lazy};
+        if (mode == 5) return {SweepChoice::SP, 1, lazy};
+        REQUIRE(c->fwd_lanes <= 1, DMT_ERR_UNSUPPORTED, "the pipelined sweep maps one lane to a (chain, block)");
+        return {SweepChoice::PIPE, 1, lazy};
+    }
+    const SweepChoice tile{SweepChoice::TILE, tile_lanes<MD, OP_SWEEP>(c, L), lazy};
+    if (mode == 1 || !eligible || c->fwd_lanes) return tile;
+    // automatic.  Warp-specialised while its grid fits ONE round of CTAs: a round costs ~0.5 ms on C3 whatever the ensemble size, so a
+    // second round loses to the one-thread-per-(chain, block) kernels (profiles/r02_tuning.md).
+    const size_t ws_units = (size_t)((c->M + 31) / 32) * L.nb;
+    if (ws_units <= (lazy ? ws_resident_ctas<MD, true>(c) : ws_resident_ctas<MD, false>(c))) return {SweepChoice::WS, 1, lazy};
+    // Then step-parallel up to 14,080 (chain, block) units: 1280 chains x 11 blocks (12 resident warps per SM at 168 registers).
+    // Measured (Lorenz, lazy noise, fused pass in ms at 512 / 1024 / 1280 chains x 10 blocks; profiles/r02_tuning.md §4e):
+    // step-parallel 0.83 / 1.10 / 1.18, two lanes per (chain, block) in the register-tile kernel 1.03 / 1.35 / 1.37.
+    if (MD::DW >= 2 && (size_t)c->M * L.nb <= 14080) return {SweepChoice::SP, 1, lazy};
+    // Then the register-tile kernel with two lanes while that grid fits one wave (1.35 against 1.40 ms for the pipelined kernel at
+    // 1024 chains, 1.03 against 1.38 ms at 512).  With the noise stored every sweep the pipelined kernel's live set (two more tile
+    // buffers) spills and it loses to the register-tile kernel (3.9 against 3.5 ms on C3); it wins where the noise is lazy (2.44 ms).
+    if (tile.lanes == 2 || !lazy) return tile;
+    return {SweepChoice::PIPE, 1, lazy};
+}
+
+template <class MD, int OP> void launch_fwd_model(dmt_ctx *c, Layout &L, FwdArgs fa) {
+    if constexpr (OP == OP_SWEEP) {
+        const SweepChoice s = pick_sweep<MD>(c, L, fa);
+        fa.lazy_w = s.lazy;
+        switch (s.kernel) {
+        case SweepChoice::TILE: launch_fwd_tile<MD, OP>(c, L, fa, s.lanes); break;
+        case SweepChoice::PIPE: s.lazy ? launch_sweep_pipe<MD, true>(c, L, fa) : launch_sweep_pipe<MD, false>(c, L, fa); break;
+        case SweepChoice::WS: s.lazy ? launch_sweep_ws<MD, true>(c, L, fa) : launch_sweep_ws<MD, false>(c, L, fa); break;
+        case SweepChoice::SP: s.lazy ? launch_sweep_sp<MD, true>(c, L, fa) : launch_sweep_sp<MD, false>(c, L, fa); break;
+        }
+        if (s.lazy) c->W_stale_layout = L.dev.id;
+    } else {
+        launch_fwd_tile<MD, OP>(c, L, fa, tile_lanes<MD, OP>(c, L));
+    }
+}
+
+template <int OP> void launch_fwd(dmt_ctx *c, Layout &L, const FwdArgs &fa) {
     // lazy noise (dmt_set_lazy_noise): an op that reads W, or rewrites only part of it, first rebuilds it from X; an op that
     // rewrites all of it just clears the flag
     if (c->W_stale_layout >= 0 && OP != OP_LOGLIK) {
@@ -452,21 +371,6 @@ template <int OP> void launch_fwd(dmt_ctx *c, Layout &L, const FwdArgs &fa_in) {
         else ensure_W(c);
     }
     ensure_guiding(c, L);
-    if (OP == OP_SWEEP) {
-        bool done = false;
-#define DMT_CASE(MID)                                                                                              \
-    case MID: done = launch_sweep_pipe<Model<MID>>(c, L, fa); break;
-        switch (c->cfg.model) {
-            DMT_FOR_MODELS(DMT_CASE)
-            default: throw DmtError(DMT_ERR_UNSUPPORTED, "model not compiled into this build of libdmt");
-        }
-#undef DMT_CASE
-        if (done) { CK(cudaGetLastError()); return; }
-    }
-    if (OP == OP_SWEEP && c->lazy_W && !fa.Z && covers_all_intervals(c, L)) { // the register-tile kernel, lazy noise: same stores skipped
-        fa.lazy_w = 1;
-        c->W_stale_layout = L.dev.id;
-    }
 #define DMT_CASE(MID)                                                                                              \
     case MID: launch_fwd_model<Model<MID>, OP>(c, L, fa); break;
     switch (c->cfg.model) {
@@ -491,7 +395,7 @@ template <class MD> void launch_bwd_model(dmt_ctx *c, Layout &L, const BwdArgs &
     for (int b = 0; b < L.nb; b++) all_terminal = all_terminal && L.last[b];
     const bool coop_ok = MD::ATIL_DIAG && MD::D >= 5 && all_terminal;
     REQUIRE(c->bwd_mode != 2 || coop_ok, DMT_ERR_UNSUPPORTED, "cooperative backward filter not available for this model / layout");
-    if (coop_ok && c->bwd_mode != 1 && !getenv("DMT_NO_COOP_K1")) {
+    if (coop_ok && c->bwd_mode != 1) {
         // wide state, no exact-observation interval: D lanes per parameter set (kernels.cuh, bwd_coop_kernel)
         constexpr int per_cta = 4 * (32 / MD::D);
         const dim3 grid((c->P + per_cta - 1) / per_cta, L.nb, nz);
@@ -802,12 +706,9 @@ int32_t dmt_create(const dmt_config *cfg, const int32_t *n_pts, const double *tt
         REQUIRE(cfg->device >= 0 && cfg->device < ndev, DMT_ERR_ARG, "device ordinal out of range");
         CK(cudaSetDevice(cfg->device));
         CK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-        {   // every lane streams whole 32-byte sectors that it alone owns (kernels.cuh): ask L2 not to promote DRAM fetches to
-            // 64/128 B, which only drags in sectors of the other accepted/proposal buffer.  DMT_L2_FETCH overrides (tuning).
-            size_t gran = 32;
-            if (const char *e = getenv("DMT_L2_FETCH")) gran = (size_t)atoi(e);
-            if (gran == 32 || gran == 64 || gran == 128) cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, gran);
-        }
+        // every lane streams whole 32-byte sectors that it alone owns (kernels.cuh): ask L2 not to promote DRAM fetches to
+        // 64/128 B, which only drags in sectors of the other accepted/proposal buffer
+        cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, 32);
 
         // ---- time grid -> tiles
         const int K = c->K;
@@ -839,7 +740,6 @@ int32_t dmt_create(const dmt_config *cfg, const int32_t *n_pts, const double *tt
         {
             bool ident = (c->P == c->M);
             for (int i = 0; i < c->M && ident; i++) ident = (pset[i] == i);
-            c->tma_ok = ident && getenv("DMT_TMA") != nullptr;
             c->pipe_ok = ident;
         }
         c->d_tile0.alloc(K + 1); c->d_step0.alloc(K + 1); c->d_pt0.alloc(K + 1); c->d_nsteps.alloc(K); c->d_ppb_tile0.alloc(K);
@@ -1548,7 +1448,7 @@ int32_t dmt_get_last_forward_kernel(dmt_ctx *ctx, char *buf, int32_t len) {
 }
 int32_t dmt_set_sweep_mode(dmt_ctx *ctx, int32_t mode) {
     return guarded(ctx, [&] {
-        if (mode < 0 || mode > 5) throw DmtError(DMT_ERR_ARG, "mode must be 0 (auto), 1 (register-tile kernel), 2 (software-pipelined kernel), 3 or 4 (warp-specialised kernel, wide / compact shape) or 5 (step-parallel kernel)");
+        if (mode < 0 || mode > 5 || mode == 4) throw DmtError(DMT_ERR_ARG, "mode must be 0 (auto), 1 (register-tile kernel), 2 (software-pipelined kernel), 3 (warp-specialised kernel) or 5 (step-parallel kernel)");
         ctx->sweep_mode = mode;
     });
 }

@@ -9,13 +9,11 @@
 // recursion starts so the stores overlap the arithmetic.
 #pragma once
 #include "kernels.cuh"
-#ifdef DMT_EXP_CLK
-#include <cstdio>
-#endif
 
 namespace dmt {
 
 // ---- TMA bulk copy + mbarrier (sm_90+): the warp-contiguous 1 KiB chunk of one component of one tile, global -> shared
+// (sweep_kernel.cuh, sweep_ws_kernel.cuh)
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t *b, int cnt) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(b)), "r"(cnt)); }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t *b, uint32_t bytes) {
@@ -29,15 +27,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t *b, uint32_t parity) {
     asm volatile("{\n.reg .pred p;\nWAIT_%=:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n@p bra DONE_%=;\nbra WAIT_%=;\nDONE_%=:\n}" ::"r"(smem_u32(b)),
                  "r"(parity) : "memory");
 }
-#ifndef DMT_HALF_TILE
-#define DMT_HALF_TILE 0 // measured: 3.61 vs 3.32 ms for the fused C3 pass (profiles/r01_tuning.md) => off
-#endif
-// 16-byte half of a lane's sector through L1: the first half-load brings the whole 32-byte sector into L1, the second one
-// (issued two steps later) hits there, so L2 still sees the sector once while only half of it is live in registers.
-__device__ __forceinline__ void ld128c(const double *p, double *v) {
-    asm volatile("ld.global.nc.v2.f64 {%0,%1}, [%2];" : "=d"(v[0]), "=d"(v[1]) : "l"(p));
-}
-constexpr int FWD_RING = 2; // tiles of H,F in flight per warp on the TMA path
 
 template <int NG> struct GTile { // where the guiding term of interval k lives for this thread's pset / law side
     const double *base;          // tile 0, component 0, this pset
@@ -62,11 +51,6 @@ __device__ __forceinline__ GTile<NG> g_tile_of(const DevCtx &cx, const LayoutDev
 // (6 CTAs of 64 threads per SM), the wider ones keep the full budget.
 // The cooperative instantiations (G > 1) only run when the GPU is far from full: no cap, no spills.
 template <class MD, int G = 1> constexpr int fwd_minb() { return G > 1 ? 1 : (DMT_FWD_MINB > 0 ? DMT_FWD_MINB : (MD::D <= 3 ? 6 : 1)); }
-#ifdef DMT_FWD_MAXREG
-#define DMT_FWD_BOUNDS __maxnreg__(DMT_FWD_MAXREG)
-#else
-#define DMT_FWD_BOUNDS __launch_bounds__(TPB, fwd_minb<MD, G>())
-#endif
 // One thread = one (chain, block).  grid = (ceil(M/TPB), n_blocks).  Replaces, per OP:
 //   OP_DRAW        draw_proposal_path!(bb)            src/biblock.jl:80-106   (pCN + guided EM + ll, fused; K3+K2+K4)
 //   OP_RECOMPUTE   recompute_path!(b°, b.WW; skip)    src/block.jl:161-187    (K2+K4)
@@ -78,19 +62,13 @@ template <class MD, int G = 1> constexpr int fwd_minb() { return G > 1 ? 1 : (DM
 //                  (docs/src/tutorials/block_collection/inference_with_blocking.md:55-57) in ONE pass over the tiles: the
 //                  accepted noise recovered by K5 feeds the pCN refresh in registers (168 instead of 264 B per step).
 //
-// TMA = true is the fast path for the common case (one pset per chain in chain order, uniform law parity): the widest stream,
-// H and F, does not go through registers at load time — per warp, lane 0 copies the NEXT tile's warp-contiguous chunks
-// (NG x 1 KiB) global -> shared with cp.async.bulk while the warp works on the current tile (2-stage ring, one mbarrier per
-// stage, no block barrier).  Measured on the memory pattern alone (profiles/r01_stream_pattern.txt): 6.3 TB/s instead of
-// 5.4 TB/s at C3's 41k threads.  All lanes of a warp stay in the loops on this path (a failed chain idles, it does not exit).
-//
 // G > 1 (ensembles too small to fill the GPU: thread count x G still fits one wave): G adjacent lanes share one
 // (chain, block).  The normals of a tile — 2 DW independent Philox + Box-Muller calls, most of the tile's instructions — are
 // split over the G lanes and all-gathered with shuffles; everything else is computed redundantly by the G lanes from the same
 // loads (one sector request per group, no extra traffic) and lane 0 of the group stores.  The random stream and every
 // result are bit-identical to G = 1.
-template <class MD, int OP, int TPB, bool TMA, int G = 1>
-__global__ void DMT_FWD_BOUNDS fwd_kernel(const DevCtx cx, const LayoutDev ly, const FwdArgs fa) {
+template <class MD, int OP, int TPB, int G = 1>
+__global__ void __launch_bounds__(TPB, fwd_minb<MD, G>()) fwd_kernel(const DevCtx cx, const LayoutDev ly, const FwdArgs fa) {
     constexpr int D = MD::D, DW = MD::DW, NPAR = MD::NPAR, NH = D * (D + 1) / 2, NG = NH + D, NAUX = D * D + D + NH;
     constexpr bool SWEEP = (OP == OP_SWEEP);
     constexpr bool READS_X = (OP == OP_LOGLIK || OP == OP_INVSOLVE || OP == OP_INVSOLVE_LL || SWEEP);
@@ -101,8 +79,8 @@ __global__ void DMT_FWD_BOUNDS fwd_kernel(const DevCtx cx, const LayoutDev ly, c
     constexpr bool WANT_LL = (OP != OP_INVSOLVE);
     constexpr bool RNG = (OP == OP_DRAW || OP == OP_INIT || SWEEP);
 
-    static_assert(G == 1 || (!TMA && (G == 2 || G == 4 || G == 8)), "lanes per chain");
-    constexpr bool UNI = TMA || (G > 1);               // warp-uniform control flow: lanes idle instead of leaving
+    static_assert(G == 1 || G == 2 || G == 4 || G == 8, "lanes per chain");
+    constexpr bool UNI = G > 1;                        // warp-uniform control flow: lanes idle instead of leaving
     const int t_raw = blockIdx.x * TPB + threadIdx.x;
     const int c_raw = t_raw / G, sub = t_raw % G;
     const int b = blockIdx.y;
@@ -142,52 +120,6 @@ __global__ void DMT_FWD_BOUNDS fwd_kernel(const DevCtx cx, const LayoutDev ly, c
     }
     double ll = 0.0, llo = 0.0;
     bool ok = true;
-#ifdef DMT_EXP_CLK // (experiment only: per-thread cycle breakdown of a tile: issue+RNG | wait+step 0 | steps 1-3 | stores)
-    long long clk_acc[4] = {0, 0, 0, 0}, ck0 = 0, ck1 = 0, ck2 = 0, ck3 = 0;
-    int clk_n = 0;
-#define DMT_CLK(v) v = clock64()
-#else
-#define DMT_CLK(v)
-#endif
-
-    // ---- TMA ring state (fast path only)
-    extern __shared__ __align__(128) unsigned char fwd_smem[];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    double *ring = reinterpret_cast<double *>(fwd_smem) + (size_t)wid * FWD_RING * NG * 128;          // [stage][component][lane][4]
-    uint64_t *bars = reinterpret_cast<uint64_t *>(fwd_smem + (size_t)(TPB / 32) * FWD_RING * NG * 1024) + wid * FWD_RING;
-    int kp = i0, qp = 0, ntl_p = 0, n_prod = 0, n_cons = 0; // producer cursor (interval, tile), tiles produced / consumed
-    const double *gp_p = nullptr;
-    uint32_t chunk_bytes = 0;
-    if (TMA) {
-        chunk_bytes = 32u * (uint32_t)min(32, cx.M - (c_raw & ~31));
-        if (lane == 0)
-            for (int s = 0; s < FWD_RING; s++) mbar_init(&bars[s], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        __syncwarp();
-        gp_p = g_tile_of<NG>(cx, ly, kp, i1, last, law_side, ps).base;
-        ntl_p = (cx.nsteps[kp] + 3) >> 2;
-    }
-    auto produce = [&]() { // every lane advances the cursor; lane 0 (always a real chain) issues the copies of its warp's chunk
-        if (kp > i1) return;
-        if (lane == 0) {
-            uint64_t *bar = &bars[n_prod % FWD_RING];
-            mbar_expect_tx(bar, NG * chunk_bytes);
-            double *dst = ring + (size_t)(n_prod % FWD_RING) * NG * 128;
-#pragma unroll
-            for (int a = 0; a < NG; a++) bulk_g2s(dst + a * 128, gp_p + ((size_t)qp * NG + a) * gstr, chunk_bytes, bar);
-        }
-        n_prod++;
-        if (++qp == ntl_p) {
-            qp = 0;
-            if (++kp <= i1) {
-                gp_p = g_tile_of<NG>(cx, ly, kp, i1, last, law_side, ps).base;
-                ntl_p = (cx.nsteps[kp] + 3) >> 2;
-            }
-        }
-    };
-    if (TMA) {
-        for (int s = 0; s < FWD_RING - 1; s++) produce();
-    }
 
     for (int k = i0; k <= i1 && (ok || SWEEP || UNI); ++k) {
         const GTile<NG> gt = g_tile_of<NG>(cx, ly, k, i1, last, law_side, ps);
@@ -234,27 +166,16 @@ __global__ void DMT_FWD_BOUNDS fwd_kernel(const DevCtx cx, const LayoutDev ly, c
         for (int q = 0; q < ntl; ++q) {
             double g[NG][4], w[DW][4], xt[D][4], dt4[4], sq4[4];
             double wo[SWEEP ? DW : 1][4], xot[SWEEP ? D : 1][4], z[RNG ? 4 * DW : 1];
-            DMT_CLK(ck0);
             // ---- every sector of the tile, once, straight into registers
             if (READS_W) {
 #pragma unroll
                 for (int j = 0; j < DW; j++) ld256(Win + ((size_t)q * DW + j) * M * 4, w[j]);
             }
-            if (TMA) produce(); // keep the copy engine FWD_RING-1 tiles ahead (the stage it refills was drained last iteration)
-            constexpr bool HALF = (DMT_HALF_TILE != 0) && !TMA; // inputs in two 16-byte halves (second half right before step 2)
-            if (!TMA) {
 #pragma unroll
-                for (int a = 0; a < NG; a++) {
-                    if (HALF) ld128c(Gp + ((size_t)q * NG + a) * gstr, g[a]);
-                    else ld256(Gp + ((size_t)q * NG + a) * gstr, g[a]);
-                }
-            }
+            for (int a = 0; a < NG; a++) ld256(Gp + ((size_t)q * NG + a) * gstr, g[a]);
             if (READS_X) {
 #pragma unroll
-                for (int i = 0; i < D; i++) {
-                    if (HALF) ld128c(Xin + ((size_t)q * D + i) * M * 4, xt[i]);
-                    else ld256(Xin + ((size_t)q * D + i) * M * 4, xt[i]);
-                }
+                for (int i = 0; i < D; i++) ld256(Xin + ((size_t)q * D + i) * M * 4, xt[i]);
             }
             ld256u(cx.dt + (size_t)(t0 + q) * 4, dt4);
             if (RNG) ld256u(cx.sqdt + (size_t)(t0 + q) * 4, sq4);
@@ -269,13 +190,8 @@ __global__ void DMT_FWD_BOUNDS fwd_kernel(const DevCtx cx, const LayoutDev ly, c
                             z[s * DW + j] = (i < nst) ? fa.Z[((size_t)(cx.step0[k] + i) * DW + j) * M + c] : 0.0;
                         }
                 } else {
-#if defined(DMT_EXP_NORNG) // (experiment only: time the kernel without the generator)
-#pragma unroll
-                    for (int s = 0; s < 4 * DW; s++) z[s] = 0.5;
-#else
                     if (G > 1) tile_normals_coop<DW, G>(cx.seed, cx.chain_offset + (uint32_t)c, (uint32_t)(t0 + q), fa.iter, (uint32_t)ly.id, sub, z);
                     else tile_normals<DW>(cx.seed, cx.chain_offset + (uint32_t)c, (uint32_t)(t0 + q), fa.iter, (uint32_t)ly.id, z);
-#endif
                 }
                 if (!SWEEP) { // K3: dW° = rho dW + sqrt(1-rho^2) sqrt(dt) xi   (A.2)
 #pragma unroll
@@ -292,21 +208,14 @@ __global__ void DMT_FWD_BOUNDS fwd_kernel(const DevCtx cx, const LayoutDev ly, c
                 }
             }
 
-            DMT_CLK(ck1);
-            const double *sg = nullptr; // TMA: this lane's sectors of the current tile in the shared-memory ring
-            if (TMA) {                  // the tile's H,F have landed; the step loop reads them in place (no register copy)
-                mbar_wait(&bars[n_cons % FWD_RING], (uint32_t)(n_cons / FWD_RING) & 1u);
-                sg = ring + (size_t)(n_cons % FWD_RING) * NG * 128 + lane * 4;
-                n_cons++;
-            }
             if (WANT_LL && k == i0 && q == 0) { // loglikhd_obs(PP[1], y1) = -c - y'Hy/2 + F'y  (src/block.jl:178)
                 double s0 = -*gt.c0;
 #pragma unroll
                 for (int i = 0; i < D; i++) {
                     double hx = 0.0;
 #pragma unroll
-                    for (int j = 0; j < D; j++) hx = fma(TMA ? sg[sidx<D>(i, j) * 128] : g[sidx<D>(i, j)][0], x[j], hx);
-                    s0 += x[i] * ((TMA ? sg[(NH + i) * 128] : g[NH + i][0]) - 0.5 * hx);
+                    for (int j = 0; j < D; j++) hx = fma(g[sidx<D>(i, j)][0], x[j], hx);
+                    s0 += x[i] * (g[NH + i][0] - 0.5 * hx);
                 }
                 ll = s0;
                 llo = s0; // same law, same start point
@@ -314,28 +223,14 @@ __global__ void DMT_FWD_BOUNDS fwd_kernel(const DevCtx cx, const LayoutDev ly, c
 #pragma unroll
             for (int s = 0; s < 4; s++) {
                 const int i = 4 * q + s;
-                if (s == 1) { DMT_CLK(ck2); }
-                if (HALF && s == 2) { // second halves of the input sectors: L1 hits
-#pragma unroll
-                    for (int a = 0; a < NG; a++) ld128c(Gp + ((size_t)q * NG + a) * gstr + 2, g[a] + 2);
-                    if (READS_X) {
-#pragma unroll
-                        for (int a = 0; a < D; a++) ld128c(Xin + ((size_t)q * D + a) * M * 4 + 2, xt[a] + 2);
-                    }
-                }
                 if (i < nst && (ok || SWEEP)) {
                     double Hs[NH], F[D], gd[D], G = 0.0;
 #pragma unroll
-                    for (int a = 0; a < NH; a++) Hs[a] = TMA ? sg[a * 128 + s] : g[a][s];
+                    for (int a = 0; a < NH; a++) Hs[a] = g[a][s];
 #pragma unroll
-                    for (int a = 0; a < D; a++) F[a] = TMA ? sg[(NH + a) * 128 + s] : g[NH + a][s];
+                    for (int a = 0; a < D; a++) F[a] = g[NH + a][s];
                     const typename MD::Diff df(par, x);
-#if defined(DMT_EXP_NOEM) // (experiment only: time the kernel without the drift / guiding arithmetic)
-#pragma unroll
-                    for (int a = 0; a < D; a++) gd[a] = Hs[a] + F[a];
-#else
                     guided_terms<MD, WANT_LL>(par, df, Bm, beta, at, Hs, F, x, gd, G);
-#endif
                     if (WANT_LL && i < nst - skip) ll = fma(G, dt4[s], ll);
                     double xn[D];
                     if (WRITES_X) { // K2: x' = x + (b + a r) dt + sigma dW   (A.3)
@@ -405,7 +300,6 @@ __global__ void DMT_FWD_BOUNDS fwd_kernel(const DevCtx cx, const LayoutDev ly, c
                     }
                 }
             }
-            DMT_CLK(ck3);
             const bool keep_w = !SWEEP || !fa.lazy_w; // lazy noise (dmt_set_lazy_noise): the blocking sweep never reads what it would store here
             if (WRITES_W && (!RNG || SWEEP) && live && keep_w) {
 #pragma unroll
@@ -423,25 +317,12 @@ __global__ void DMT_FWD_BOUNDS fwd_kernel(const DevCtx cx, const LayoutDev ly, c
 #pragma unroll
                 for (int i = 0; i < D; i++) st256(Xout + ((size_t)q * D + i) * M * 4, xt[i]);
             }
-#ifdef DMT_EXP_CLK
-            { long long ck4 = clock64(); clk_acc[0] += ck1 - ck0; clk_acc[1] += ck2 - ck1; clk_acc[2] += ck3 - ck2; clk_acc[3] += ck4 - ck3; clk_n++; }
-#endif
-            if (TMA) __syncwarp(); // every lane is done with this stage: the next produce() may refill it
             if (!ok && !SWEEP && !UNI) break;
         }
     }
-#ifdef DMT_EXP_CLK
-    if (SWEEP && (c % 1024) == 37 && (b == 2 || b == 7) && fa.iter == 9)
-        printf("CLK c=%d b=%d tiles=%d  issue+rng %lld  wait+step0 %lld  steps1-3 %lld  stores %lld (cycles per tile)\n", c, b, clk_n, clk_acc[0] / clk_n,
-               clk_acc[1] / clk_n, clk_acc[2] / clk_n, clk_acc[3] / clk_n);
-#endif
     if (WANT_LL && live) ly.ll[((size_t)ll_side * ly.nb + b) * M + c] = ll;
     if (SWEEP && live) ly.ll[((size_t)ly.nb + b) * M + c] = llo;
     if ((WRITES_X || SWEEP) && live) ly.ok[(size_t)b * M + c] = ok ? 1 : 0;
-}
-
-template <class MD, int TPB, bool TMA> constexpr size_t fwd_smem_bytes() {
-    return TMA ? (size_t)(TPB / 32) * FWD_RING * (MD::D * (MD::D + 1) / 2 + MD::D) * 1024 + (size_t)(TPB / 32) * FWD_RING * 8 : 0;
 }
 
 } // namespace dmt

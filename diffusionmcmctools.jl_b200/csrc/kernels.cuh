@@ -27,9 +27,6 @@ namespace dmt {
 #ifndef DMT_FWD_MINB
 #define DMT_FWD_MINB 0 // min resident CTAs per SM promised to ptxas (caps registers); 0 = per-model default (fwd_minb)
 #endif
-#ifndef DMT_EVICT_FIRST
-#define DMT_EVICT_FIRST 1 // 1: streamed sectors are marked L2::evict_first (spill lines and per-interval records stay in L2)
-#endif
 #ifndef DMT_BWD_MINB
 #define DMT_BWD_MINB 1
 #endif
@@ -101,30 +98,15 @@ struct FwdArgs {
 };
 
 // ------------------------------------------------------------------------------------------- 256-bit sector access
+// streamed sectors are marked L2::evict_first: spill lines and per-interval records stay in L2
 __device__ __forceinline__ void ld256(const double *p, double *v) { // streaming read-only sector
-#if defined(DMT_LD256_SPLIT) // (experiment: the sector as two 128-bit loads)
-    asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0,%1}, [%2];" : "=d"(v[0]), "=d"(v[1]) : "l"(p));
-    asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0,%1}, [%2];" : "=d"(v[2]), "=d"(v[3]) : "l"(p + 2));
-#elif DMT_EVICT_FIRST
     asm volatile("ld.global.nc.L1::no_allocate.L2::evict_first.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(v[0]), "=d"(v[1]), "=d"(v[2]), "=d"(v[3]) : "l"(p));
-#else
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(v[0]), "=d"(v[1]), "=d"(v[2]), "=d"(v[3]) : "l"(p));
-#endif
 }
 __device__ __forceinline__ void ld256u(const double *p, double *v) { // chain-uniform data (dt, sqrt dt): keep in L1
-#if defined(DMT_DT_SCALAR)
-    const double2 a = __ldg(reinterpret_cast<const double2 *>(p)), b = __ldg(reinterpret_cast<const double2 *>(p) + 1);
-    v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y;
-#else
     asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(v[0]), "=d"(v[1]), "=d"(v[2]), "=d"(v[3]) : "l"(p));
-#endif
 }
 __device__ __forceinline__ void st256(double *p, const double *v) {
-#if DMT_EVICT_FIRST
     asm volatile("st.global.L1::no_allocate.L2::evict_first.v4.f64 [%4], {%0,%1,%2,%3};" ::"d"(v[0]), "d"(v[1]), "d"(v[2]), "d"(v[3]), "l"(p) : "memory");
-#else
-    asm volatile("st.global.L1::no_allocate.v4.f64 [%4], {%0,%1,%2,%3};" ::"d"(v[0]), "d"(v[1]), "d"(v[2]), "d"(v[3]), "l"(p) : "memory");
-#endif
 }
 __device__ __forceinline__ void prefetch_l2(const void *p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 

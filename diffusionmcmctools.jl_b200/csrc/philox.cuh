@@ -71,19 +71,6 @@ __device__ __forceinline__ void tile_normals(uint64_t seed, uint32_t chain, uint
     }
 }
 
-// normal number n (0 .. 4*DW-1) of a tile, generated on demand: even n evaluates Philox call n/2 and keeps its second normal in
-// `carry` for n+1 (same values as tile_normals; at most one spare normal is live instead of the whole tile's 4*DW)
-template <int N>
-__device__ __forceinline__ double tile_normal_at(uint64_t seed, uint32_t chain, uint32_t gtile, uint32_t iter, uint32_t layout, double &carry) {
-    if ((N & 1) == 0) {
-        double z0;
-        u32x4 c = {chain, gtile, iter, ctr_word3(STREAM_PCN, layout, (uint32_t)(N / 2))};
-        box_muller(philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32)), z0, carry);
-        return z0;
-    }
-    return carry;
-}
-
 // the same 4*DW normals, produced by G adjacent lanes together: lane `sub` of the group evaluates calls sub, sub+G, ... and the
 // group all-gathers the pairs with shuffles (every lane of the warp must call this)
 template <int DW, int G>

@@ -47,14 +47,9 @@ template <class MD> constexpr size_t sweep_pipe_smem() {
     return (size_t)2 * (NG * 128 + 8) * 8 + (size_t)(D * D + D) * 32 * 8 + 2 * 8;
 }
 
-// G > 1 (ensembles too small to give every scheduler a warp: 512 chains x 10 blocks are 168 warps on 592 schedulers): G adjacent
-// lanes share one (chain, block).  They split the tile's 2 DW Philox + Box-Muller calls and all-gather the normals with shuffles
-// (philox.cuh, tile_normals_coop); everything else is computed redundantly from the same shared-memory sectors and lane 0 of the group
-// stores.  Random stream and results are bit-identical to G = 1.
-template <class MD, bool LAZYW, int G = 1>
+// One lane per (chain, block), 32 chains per warp.
+template <class MD, bool LAZYW>
 __global__ void __launch_bounds__(32, sweep_pipe_minb<MD>()) sweep_pipe_kernel(const DevCtx cx, const LayoutDev ly, const FwdArgs fa) {
-    static_assert(G == 1 || G == 2 || G == 4 || G == 8, "lanes per (chain, block)");
-    constexpr int CPW = 32 / G; // chains per warp
     constexpr int D = MD::D, DW = MD::DW, NPAR = MD::NPAR, NH = D * (D + 1) / 2, NG = NH + D, NAUX = D * D + D + NH;
     constexpr int STAGE = NG * 128 + 8; // doubles per stage: [component][lane][4] then dt[4], sqrt(dt)[4]
     extern __shared__ __align__(128) unsigned char sw_smem[];
@@ -62,18 +57,18 @@ __global__ void __launch_bounds__(32, sweep_pipe_minb<MD>()) sweep_pipe_kernel(c
     double *cst = ring + 2 * STAGE;                                  // [D*D + D][32]: B (row-major), beta of the current interval
     uint64_t *bars = reinterpret_cast<uint64_t *>(cst + (D * D + D) * 32);
 
-    const int lane = threadIdx.x, cl = lane / G, sub = lane % G; // chain slot inside the warp, lane inside the chain's group
-    const int c0 = blockIdx.x * CPW, b = blockIdx.y;
+    const int lane = threadIdx.x;
+    const int c0 = blockIdx.x * 32, b = blockIdx.y;
     if (c0 >= cx.M) return;
-    const int c_raw = c0 + cl;
+    const int c_raw = c0 + lane;
     const int c = min(c_raw, cx.M - 1); // lanes beyond the ensemble shadow the last chain and never store
-    const bool live = c_raw < cx.M && sub == 0;
+    const bool live = c_raw < cx.M;
     const size_t M = cx.M, P = cx.P;
     const int ps = c;                   // launch condition: one parameter set per chain, in chain order
     const int i0 = ly.i0[b], i1 = ly.i1[b];
     const bool last = ly.last[b] != 0;
     const double rho = ly.rho[b], crho = sqrt(1.0 - rho * rho);
-    const uint32_t chunk_bytes = 32u * (uint32_t)min(CPW, cx.M - c0);
+    const uint32_t chunk_bytes = 32u * (uint32_t)min(32, cx.M - c0);
     const size_t gstr = P * 4;
 
     if (lane == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); }
@@ -82,17 +77,13 @@ __global__ void __launch_bounds__(32, sweep_pipe_minb<MD>()) sweep_pipe_kernel(c
 
     // ---- prefetch cursor: the tile after the one being computed
     int kn = i0, qn = 0, ntl_n = (cx.nsteps[i0] + 3) >> 2, t0_n = cx.tile0[i0], n_prod = 0;
-    const double *gp_n = g_tile_of<NG>(cx, ly, i0, i1, last, 0, c0).base; // warp-uniform: the chunk of chain c0's lane group
+    const double *gp_n = g_tile_of<NG>(cx, ly, i0, i1, last, 0, c0).base; // warp-uniform: the chunk of the warp's first chain
     const double *xin_n = cx.X + (size_t)cx.parX[(size_t)i0 * M + c] * cx.Xbuf + ((size_t)t0_n * D * M + c) * 4;
     bool more = true;
     double xnx[D][4];
     auto prefetch = [&]() { // issue every load of tile (kn, qn), then advance the cursor
         if (!more) return;
-#ifdef DMT_SW_LANE0_ISSUE
-        if (lane == 0) {
-#else
         if (elect_one_lane()) {
-#endif
             uint64_t *bar = &bars[n_prod & 1];
             double *dst = ring + (size_t)(n_prod & 1) * STAGE;
             mbar_expect_tx(bar, NG * chunk_bytes + 64u);
@@ -168,7 +159,6 @@ __global__ void __launch_bounds__(32, sweep_pipe_minb<MD>()) sweep_pipe_kernel(c
 #pragma unroll
                 for (int s = 0; s < 4; s++) xt[i][s] = xnx[i][s];
             prefetch(); // tile t+1: its stage was drained at the end of tile t-1 (the __syncwarp below)
-#ifndef DMT_SW_NO_PFREC
             if (q == ntl - 1 && k < i1) { // the next interval's law records and start point: pull them into L2 one tile ahead, so that the
                                           // dependent loads at the interval boundary do not pay a DRAM round trip each (ncu: 12 % of all stall samples)
                 const int k1 = k + 1;
@@ -188,17 +178,14 @@ __global__ void __launch_bounds__(32, sweep_pipe_minb<MD>()) sweep_pipe_kernel(c
                 prefetch_l2(cx.parX + (size_t)k1 * M + c);
                 prefetch_l2(cx.parW + (size_t)k1 * M + c);
             }
-#endif
-#ifndef DMT_SW_ZONDEMAND // the tile's normals BEFORE the wait for its data: the generator runs while the sectors are still in flight
+            // the tile's normals BEFORE the wait for its data: the generator runs while the sectors are still in flight
             // (measured, profiles/r02_tuning.md: 2.44 ms against 2.61-3.08 ms with the normals generated inside the step loop)
             double z[4 * DW];
-            if (G > 1) tile_normals_coop<DW, G>(cx.seed, cx.chain_offset + (uint32_t)c, (uint32_t)(t0 + q), fa.iter, (uint32_t)ly.id, sub, z);
-            else tile_normals<DW>(cx.seed, cx.chain_offset + (uint32_t)c, (uint32_t)(t0 + q), fa.iter, (uint32_t)ly.id, z);
-#endif
+            tile_normals<DW>(cx.seed, cx.chain_offset + (uint32_t)c, (uint32_t)(t0 + q), fa.iter, (uint32_t)ly.id, z);
 
             mbar_wait(&bars[n_cons & 1], (uint32_t)(n_cons >> 1) & 1u);
             const double *st = ring + (size_t)(n_cons & 1) * STAGE;
-            const double *sg = st + cl * 4;
+            const double *sg = st + lane * 4;
             n_cons++;
             if (k == i0 && q == 0) { // loglikhd_obs(PP[1], y1) = -c - y'Hy/2 + F'y  (src/block.jl:178)
                 double s0 = -*gt.c0;
@@ -212,7 +199,7 @@ __global__ void __launch_bounds__(32, sweep_pipe_minb<MD>()) sweep_pipe_kernel(c
                 ll = s0;
                 llo = s0; // same law, same start point
             }
-            double w[LAZYW ? 1 : DW][4], wo[LAZYW ? 1 : DW][4], xot[D][4], zcarry = 0.0;
+            double w[LAZYW ? 1 : DW][4], wo[LAZYW ? 1 : DW][4], xot[D][4];
             // One EM step of the tile.  FULL (every step of the tile exists — always, on grids whose intervals hold a multiple of 4
             // steps): no branch at all, so the four steps and the generator calls they consume form ONE basic block that ptxas can
             // interleave; a failed proposal keeps computing (its state is unspecified anyway) and is marked at the end.
@@ -222,17 +209,10 @@ __global__ void __launch_bounds__(32, sweep_pipe_minb<MD>()) sweep_pipe_kernel(c
                 const int i = 4 * q + s;
                 if (FULL || i < nst) {
                     double Hs[NH], F[D], Bm[D * D], beta[D], gd[D], G = 0.0;
-#ifdef DMT_SWEXP_NOCONF // (experiment only: bank-conflict-free reads of the WRONG elements, to price the 32-byte lane stride)
-#pragma unroll
-                    for (int a = 0; a < NH; a++) Hs[a] = st[a * 128 + s * 32 + lane];
-#pragma unroll
-                    for (int a = 0; a < D; a++) F[a] = st[(NH + a) * 128 + s * 32 + lane];
-#else
 #pragma unroll
                     for (int a = 0; a < NH; a++) Hs[a] = sg[a * 128 + s];
 #pragma unroll
                     for (int a = 0; a < D; a++) F[a] = sg[(NH + a) * 128 + s];
-#endif
 #pragma unroll
                     for (int a = 0; a < D * D; a++) Bm[a] = cst[a * 32 + lane];
 #pragma unroll
@@ -250,16 +230,9 @@ __global__ void __launch_bounds__(32, sweep_pipe_minb<MD>()) sweep_pipe_kernel(c
 #pragma unroll
                     for (int a = 0; a < D; a++) x[a] = xn[a];
                     double dwo[DW];
-                    static_for<DW>([&](auto j_c) { // K3: dW° = rho dW + sqrt(1-rho^2) sqrt(dt) xi   (A.2); xi generated as it is needed
+                    static_for<DW>([&](auto j_c) { // K3: dW° = rho dW + sqrt(1-rho^2) sqrt(dt) xi   (A.2)
                         constexpr int j = decltype(j_c)::value;
-#ifdef DMT_SWEXP_NORNG // (experiment only: the pass without the generator)
-                        const double xi = 0.5 + zcarry;
-#elif !defined(DMT_SW_ZONDEMAND)
                         const double xi = z[s * DW + j];
-                        (void)zcarry;
-#else
-                        const double xi = tile_normal_at<s * DW + j>(cx.seed, cx.chain_offset + (uint32_t)c, (uint32_t)(t0 + q), fa.iter, (uint32_t)ly.id, zcarry);
-#endif
                         dwo[j] = rho * dwv[j] + crho * sq * xi;
                         if (!LAZYW) { w[j][s] = dwv[j]; wo[j][s] = dwo[j]; }
                     });
@@ -290,11 +263,7 @@ __global__ void __launch_bounds__(32, sweep_pipe_minb<MD>()) sweep_pipe_kernel(c
                     }
                 }
             };
-#ifdef DMT_SW_NOFULL
-            if (false) {}
-#else
             if (4 * q + 4 <= nst) static_for<4>([&](auto s_c) { step(s_c, std::true_type{}); });
-#endif
             else static_for<4>([&](auto s_c) { step(s_c, std::false_type{}); });
             if (live) {
                 if (!LAZYW) {

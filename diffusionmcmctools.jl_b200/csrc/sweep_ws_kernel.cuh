@@ -33,37 +33,19 @@
 // kernels' up to FP64 rounding (a different summation / FMA contraction order); the random stream is bit-identical.
 #pragma once
 #include "sweep_kernel.cuh"
-#include <new>
 #ifdef DMT_WS_TRACE
 #include <cstdio>
 #endif
 
-#ifndef DMT_WSC_LUNROLL // compact shape: passes of the L warp interleaved per loop trip (instruction-level parallelism for a lone warp)
-#define DMT_WSC_LUNROLL 1
-#endif
-#ifndef DMT_WSC_RUNROLL // compact shape: generator calls interleaved per loop trip
-#define DMT_WSC_RUNROLL 1
-#endif
-
-#ifndef DMT_WSC_LUNROLL // compact shape: passes of the L warp interleaved per loop trip (instruction-level parallelism for a lone warp)
-#define DMT_WSC_LUNROLL 1
-#endif
-#ifndef DMT_WSC_RUNROLL // compact shape: generator calls interleaved per loop trip
-#define DMT_WSC_RUNROLL 1
-#endif
-
 namespace dmt {
-constexpr int WSC_LUNROLL = DMT_WSC_LUNROLL, WSC_RUNROLL = DMT_WSC_RUNROLL;
 
-// Two shapes.  WIDE (16 warps: P, T, up to 6 R, 4 A, 4 L): the shortest time per tile, but 16 warps x 128 registers fill an SM's
-// register file — one CTA per SM.  COMPACT (8 warps: P, 2 R, 4 A and ONE warp that does the four L passes of a tile and issues the TMA
-// copies): a little slower per tile, two CTAs per SM — for grids of more units than SMs, where the wide shape would need a second round.
-template <int NR_, int NSG_, int NSR_, bool COMPACT_ = false> struct WsShape {
-    static constexpr bool COMPACT = COMPACT_;
-    static constexpr int NR = NR_, NA = 4, NL = COMPACT ? 1 : 4, NSG = NSG_, NSZ = NSR_, NSD = NSR_, NSX = NSR_;
-    static constexpr int WARPS = COMPACT ? 8 : 16, THREADS = WARPS * 32;
+// 16 warps (P, T, up to 6 R, 4 A, 4 L): 16 warps x 128 registers fill an SM's register file — one CTA per SM.  NR generator warps,
+// NSG stages of the G ring, NSR slots of each of the Z, D and X rings.
+template <int NR_, int NSG_, int NSR_> struct WsShape {
+    static constexpr int NR = NR_, NA = 4, NL = 4, NSG = NSG_, NSZ = NSR_, NSD = NSR_, NSX = NSR_;
+    static constexpr int WARPS = 16, THREADS = WARPS * 32;
     static constexpr int NBAR = 2 * (NSG + NSZ + NSD + NSX);
-    static_assert(COMPACT ? NR == 2 : (NR >= 1 && NR <= 6), "generator warps: 2 in the compact shape, up to 6 in the wide one");
+    static_assert(NR >= 1 && NR <= 6, "generator warps: up to 6");
 };
 constexpr int WS_RS = 36; // row stride of the Z / D / X rings in doubles
 // step stride of the transposed guiding term inside a D-ring slot: >= NG rows, and = 4 (mod 16) so that the (chain, step) writers
@@ -71,13 +53,8 @@ constexpr int WS_RS = 36; // row stride of the Z / D / X rings in doubles
 __host__ __device__ constexpr int ws_gt_stride(int NG) { int v = NG * WS_RS; while (v % 16 != 4) v += 4; return v; }
 // Warp -> role.  Warp w issues on scheduler w % 4.  The recursion warp P shares its scheduler only with the lightest warps (the TMA
 // lane and two L warps); the generator warps, which saturate the FP64 pipe of their scheduler, are spread over the other three.
-enum { WS_P = 0, WS_T = 1, WS_R = 2, WS_A = 3, WS_L = 4, WS_LT = 5 };
-template <bool COMPACT> __device__ __forceinline__ void ws_role_of(int warp, int &role, int &id) {
-    if (COMPACT) { // w: 0 P | 1, 2 R | 3 L + T | 4..7 A
-        role = warp == 0 ? WS_P : warp <= 2 ? WS_R : warp == 3 ? WS_LT : WS_A;
-        id = warp == 0 ? 0 : warp <= 2 ? warp - 1 : warp == 3 ? 0 : warp - 4;
-        return;
-    }
+enum { WS_P = 0, WS_T = 1, WS_R = 2, WS_A = 3, WS_L = 4 };
+__device__ __forceinline__ void ws_role_of(int warp, int &role, int &id) {
     // w:      15 14 13 12 11 10  9  8  7  6  5  4  3  2  1  0      (one hex digit per warp; no table in local memory)
     // role:    A  L  L  L  A  A  A  L  R  R  R  T  R  R  R  P
     // id:      3  3  2  1  2  1  0  0  5  4  3  0  2  1  0  0
@@ -85,15 +62,11 @@ template <bool COMPACT> __device__ __forceinline__ void ws_role_of(int warp, int
     id = (int)((0x3321210054302100ull >> (4 * warp)) & 0xfull);
 }
 
-// (compact shape) the law record of the current interval for the CTA's 32 chains: the model's Par as raw doubles, B, beta [, atilde]
-template <class MD> __host__ __device__ constexpr int ws_law_fields() {
-    return (int)(sizeof(typename MD::Par) / 8) + MD::D * MD::D + MD::D + (MD::CONSTDIFF ? 0 : MD::D * (MD::D + 1) / 2);
-}
 template <class MD, class SH> constexpr size_t sweep_ws_smem() {
     constexpr int D = MD::D, DW = MD::DW, NG = D * (D + 1) / 2 + D;
     return (size_t)SH::NSG * (NG * 128 + 8) * 8 + (size_t)SH::NSZ * (4 * DW) * WS_RS * 8 +
            (size_t)SH::NSD * ((4 * DW) * WS_RS + 4 * ws_gt_stride(NG)) * 8 + (size_t)SH::NSX * 5 * D * WS_RS * 8 + (size_t)3 * 32 * 8 + SH::NBAR * 8 +
-           (size_t)(D * D + D) * 32 * 8 + (SH::COMPACT ? (size_t)(ws_law_fields<MD>() + 4) * 32 * 8 : 0);
+           (size_t)(D * D + D) * 32 * 8;
 }
 
 __device__ __forceinline__ void mbar_arrive(uint64_t *b) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(b)) : "memory"); }
@@ -111,8 +84,8 @@ struct WsCursor { // (interval, tile inside it) of a tile of the block
     int k, q, ntl, t0;
 };
 
-template <class MD, bool LAZYW, class SH, int MINB>
-__global__ void __launch_bounds__(SH::THREADS, MINB) sweep_ws_kernel(const DevCtx cx, const LayoutDev ly, const FwdArgs fa) {
+template <class MD, bool LAZYW, class SH>
+__global__ void __launch_bounds__(SH::THREADS, 1) sweep_ws_kernel(const DevCtx cx, const LayoutDev ly, const FwdArgs fa) {
     constexpr int NR = SH::NR, NA = SH::NA, NL = SH::NL, NSG = SH::NSG, NSZ = SH::NSZ, NSD = SH::NSD, NSX = SH::NSX, RS = WS_RS;
     constexpr int D = MD::D, DW = MD::DW, NPAR = MD::NPAR, NH = D * (D + 1) / 2, NG = NH + D, NAUX = D * D + D + NH;
     constexpr int STAGE = NG * 128 + 8, NZ = 4 * DW, ZS = NZ * RS, XS = 5 * D * RS, SS = ws_gt_stride(NG), DS = ZS + 4 * SS;
@@ -126,11 +99,10 @@ __global__ void __launch_bounds__(SH::THREADS, MINB) sweep_ws_kernel(const DevCt
     uint64_t *full_g = bars, *empty_g = full_g + NSG, *full_z = empty_g + NSG, *empty_z = full_z + NSZ;
     uint64_t *full_d = empty_z + NSZ, *empty_d = full_d + NSD, *full_x = empty_d + NSD, *empty_x = full_x + NSX;
     double *alaw = reinterpret_cast<double *>(empty_x + NSX);    // [D*D + D][32]: B, beta of the A warps' chains for the current interval
-    double *lawbuf = alaw + (D * D + D) * 32;                      // (compact) [ws_law_fields][32], then the L warp's accumulators [4][32]
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     int role, w_id;
-    ws_role_of<SH::COMPACT>(warp, role, w_id);
+    ws_role_of(warp, role, w_id);
     const int c0 = blockIdx.x * 32, b = blockIdx.y;
     if (c0 >= cx.M) return;
     const size_t M = cx.M, P = cx.P;
@@ -311,7 +283,7 @@ __global__ void __launch_bounds__(SH::THREADS, MINB) sweep_ws_kernel(const DevCt
             wait_empty(empty_z, j, NSZ);
             WS_TR(j, 1)
             double *zo = zring + (size_t)(j % NSZ) * ZS + lane;
-#pragma unroll(SH::COMPACT ? WSC_RUNROLL : 1)
+#pragma unroll 1
             for (int call = r; call < 2 * DW; call += NR) {
                 u32x4 ctr = {cx.chain_offset + (uint32_t)c, (uint32_t)(u.t0 + u.q), fa.iter, ctr_word3(STREAM_PCN, (uint32_t)ly.id, (uint32_t)call)};
                 double z0, z1;
@@ -324,149 +296,6 @@ __global__ void __launch_bounds__(SH::THREADS, MINB) sweep_ws_kernel(const DevCt
             cur_next(u);
         }
         WS_TR_DUMP("R")
-        }
-    } else if (role == WS_LT) {
-        // ================================================================== L + T (compact shape): the four L passes of every tile in one
-        // warp, the law record staged in shared memory once per interval (lane = chain, coalesced), and the TMA producer of the G ring
-        // on lane 0.  L is the LAST consumer of a stage, so the stage of tile j is free the moment this warp has released it: tile
-        // j + NSG is issued right there (A runs at most NSD + NSX + 2 tiles ahead of L, so the copies still have NSG - that many tiles to land).
-        constexpr int NPD = (int)(sizeof(typename MD::Par) / 8), NF = ws_law_fields<MD>();
-        union ParU { typename MD::Par p; double d[NPD]; __device__ ParU() {} };
-        double *lacc = lawbuf + NF * 32;
-        const int s = lane & 3;
-        const int cs = min(c0 + lane, cx.M - 1);
-        auto stage_law = [&](int k) {
-            int slot, store;
-            law_of(k, cs, slot, store);
-            double th[NPAR];
-            const double *tp = cx.theta[slot][store] + (size_t)k * NPAR * P + cs;
-#pragma unroll
-            for (int i = 0; i < NPAR; i++) th[i] = tp[(size_t)i * P];
-            ParU w;
-            new (&w.p) typename MD::Par(th);
-            __syncwarp(); // every lane is done reading the previous interval's record
-#pragma unroll
-            for (int i = 0; i < NPD; i++) lawbuf[i * 32 + lane] = w.d[i];
-            const double *ap = cx.aux[slot][store] + (size_t)k * NAUX * P + cs;
-#pragma unroll
-            for (int i = 0; i < NF - NPD; i++) lawbuf[(NPD + i) * 32 + lane] = ap[(size_t)i * P];
-            if (k < i1) {
-                int slot1, store1;
-                law_of(k + 1, cs, slot1, store1);
-                const double *tp1 = cx.theta[slot1][store1] + (size_t)(k + 1) * NPAR * P + cs;
-                const double *ap1 = cx.aux[slot1][store1] + (size_t)(k + 1) * NAUX * P + cs;
-#pragma unroll
-                for (int i = 0; i < NPAR; i++) prefetch_l2(tp1 + (size_t)i * P);
-#pragma unroll
-                for (int i = 0; i < NF - NPD; i++) prefetch_l2(ap1 + (size_t)i * P);
-            }
-            __syncwarp();
-        };
-        WsCursor tc = cur_init();
-        int jt = 0, k_cur = -1;
-        const double *gp = nullptr;
-        auto issue = [&]() { // the TMA copies of tile jt (lane 0); the cursor advances on every lane
-            if (jt >= T) return;
-            if (lane == 0) {
-                if (tc.k != k_cur) { gp = g_tile_of<NG>(cx, ly, tc.k, i1, last, 0, c0).base; k_cur = tc.k; }
-                wait_empty(empty_g, jt, NSG);
-                uint64_t *bar = &full_g[jt % NSG];
-                double *dst = gring + (size_t)(jt % NSG) * STAGE;
-                mbar_expect_tx(bar, NG * chunk_bytes + 64u);
-#pragma unroll 1
-                for (int a = 0; a < NG; a++) bulk_g2s(dst + a * 128, gp + ((size_t)tc.q * NG + a) * gstr, chunk_bytes, bar);
-                bulk_g2s(dst + NG * 128, cx.dt + (size_t)(tc.t0 + tc.q) * 4, 32u, bar);
-                bulk_g2s(dst + NG * 128 + 4, cx.sqdt + (size_t)(tc.t0 + tc.q) * 4, 32u, bar);
-            }
-            jt++;
-            cur_next(tc);
-        };
-        for (int i = 0; i < NSG; i++) issue();
-#pragma unroll
-        for (int p = 0; p < 4; p++) lacc[p * 32 + lane] = 0.0;
-        WsCursor u = cur_init();
-        int k_loaded = -1, nst = 0;
-        unsigned bad = 0u; // bit p: this lane's (chain, step) of pass p has failed
-        WS_TR_DECL
-        for (int j = 0; j < T; j++) {
-            WS_TR(j, 0)
-            if (u.k != k_loaded) {
-                stage_law(u.k);
-                nst = cx.nsteps[u.k];
-                k_loaded = u.k;
-            }
-            const bool on = 4 * u.q + s < nst;
-            wait_full(full_g, j, NSG);
-            const double *st = gring + (size_t)(j % NSG) * STAGE;
-            const double dt = st[NG * 128 + s];
-            wait_full(full_x, j, NSX);
-            WS_TR(j, 1)
-            const double *xs0 = xring + (size_t)(j % NSX) * XS;
-#pragma unroll WSC_LUNROLL
-            for (int p = 0; p < 4; p++) {
-                const int cl = 8 * p + (lane >> 2);
-                const double *sg = st + p * 32 + lane;
-                const double *xs = xs0 + cl;
-                ParU pu;
-                double Bm[D * D], beta[D], at[NH], Hs[NH], F[D], xb[D], xn[D], gdo[D], Go = 0.0;
-#pragma unroll
-                for (int i = 0; i < NPD; i++) pu.d[i] = lawbuf[i * 32 + cl];
-#pragma unroll
-                for (int i = 0; i < D * D; i++) Bm[i] = lawbuf[(NPD + i) * 32 + cl];
-#pragma unroll
-                for (int i = 0; i < D; i++) beta[i] = lawbuf[(NPD + D * D + i) * 32 + cl];
-                if (!MD::CONSTDIFF) {
-#pragma unroll
-                    for (int i = 0; i < NH; i++) at[i] = lawbuf[(NPD + D * D + D + i) * 32 + cl];
-                }
-#pragma unroll
-                for (int a = 0; a < NH; a++) Hs[a] = sg[a * 128];
-#pragma unroll
-                for (int a = 0; a < D; a++) F[a] = sg[(NH + a) * 128];
-#pragma unroll
-                for (int a = 0; a < D; a++) { xb[a] = xs[(a * 5 + s) * RS]; xn[a] = xs[(a * 5 + s + 1) * RS]; }
-                const typename MD::Par &par = pu.p;
-                const typename MD::Diff dfo(par, xb);
-                guided_terms<MD, true>(par, dfo, Bm, beta, at, Hs, F, xb, gdo, Go);
-                double acc = lacc[p * 32 + lane];
-                if (j == 0 && s == 0) { // the same start term as the accepted path: same law, same start point (src/block.jl:178)
-                    const GTile<NG> gt = g_tile_of<NG>(cx, ly, i0, i1, last, 0, min(c0 + cl, cx.M - 1));
-                    double s0 = -*gt.c0;
-#pragma unroll
-                    for (int i = 0; i < D; i++) {
-                        double hx = 0.0;
-#pragma unroll
-                        for (int jj = 0; jj < D; jj++) hx = fma(Hs[sidx<D>(i, jj)], xb[jj], hx);
-                        s0 += xb[i] * (F[i] - 0.5 * hx);
-                    }
-                    acc = s0;
-                }
-                if (on) {
-                    acc = fma(Go, dt, acc);
-                    bool fin = dfo.ok();
-#pragma unroll
-                    for (int a = 0; a < D; a++) fin = fin && isfinite(xn[a]);
-                    if (!(fin && MD::bound_ok(par, xn))) bad |= 1u << p; // src/block.jl:181 (ll° := -Inf once, after the loop)
-                }
-                lacc[p * 32 + lane] = acc;
-            }
-            signal(empty_x, j, NSX);
-            signal(empty_g, j, NSG);
-            issue(); // tile j + NSG into the stage just released
-            WS_TR(j, 2)
-            cur_next(u);
-        }
-        WS_TR_DUMP("L")
-#pragma unroll
-        for (int p = 0; p < 4; p++) {
-            double v = lacc[p * 32 + lane];
-            v += __shfl_xor_sync(0xffffffffu, v, 1);
-            v += __shfl_xor_sync(0xffffffffu, v, 2);
-            const unsigned b4 = __ballot_sync(0xffffffffu, (bad >> p) & 1u);
-            if (s == 0) {
-                part[32 + 8 * p + (lane >> 2)] = v;
-                part[64 + 8 * p + (lane >> 2)] = ((b4 >> (lane & ~3)) & 0xfu) ? 0.0 : 1.0;
-            }
         }
     } else {
         // ================================================================== A and L: one lane per (chain, step), 8 chains per warp

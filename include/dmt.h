@@ -216,27 +216,32 @@ int32_t dmt_enable_guiding_cache(dmt_ctx *ctx, int32_t layout, int32_t enable);
 /* accepted-side guiding term as ops on `layout` see it (the layout-private store when the cache is valid, else the shared one) */
 int32_t dmt_get_layout_guiding_term(dmt_ctx *ctx, int32_t layout, int32_t store, int32_t k, double *H, double *F, double *c);
 
-/* ---- tuning: lanes per (chain, block) in the forward kernel (K2-K5) ------------------------------------------------
+/* ---- tuning: lanes per (chain, block) in the register-tile forward kernel (K2-K5) ------------------------------------
  * 0 (default) = automatic: 1 lane when chains x blocks fill the GPU, else the largest of 2/4/8 for which all threads are still
  * resident at once — the lanes split the tile's Philox/Box-Muller calls and compute everything else redundantly, so results
- * and random streams are bit-identical for every setting.  1, 2, 4, 8 force a value.  No counterpart in the reference (its
- * per-recording loop, src/block_ensemble.jl:50, is serial). */
+ * and random streams are bit-identical for every setting.  1, 2, 4, 8 force a value; under dmt_set_sweep_mode(0) a forced value
+ * also makes the fused sweep pass run the register-tile kernel.  No counterpart in the reference (its per-recording loop,
+ * src/block_ensemble.jl:50, is serial). */
 int32_t dmt_set_fwd_lanes(dmt_ctx *ctx, int32_t lanes);
 
 /* ---- tuning: memory schedule of the fused blocking-sweep pass (dmt_blocking_sweep / dmt_find_W_loglikhd_draw) ----------
- * 0 (default) = automatic: the software-pipelined kernel (guiding term through a TMA shared-memory ring, X double-buffered in
- * registers; sweep_kernel.cuh) when every chain owns its parameter set in chain order, the law parity is uniform, Z == NULL and
- * dmt_set_fwd_lanes is automatic; the register-tile kernel otherwise.  1 = always the register-tile kernel.  2 = pipelined kernel or
- * DMT_ERR_UNSUPPORTED.  3 / 4 = warp-specialised kernel (sweep_ws_kernel.cuh: per group of 32 chains and block a CTA whose
- * warps form a pipeline — TMA producer, generator warps, inverse solve + accepted likelihood, the proposal's recursion, the proposal's
- * likelihood — over shared-memory rings) in its wide (16 warps, one CTA per SM) / compact (8 warps, two per SM) shape, under the same
- * conditions, or DMT_ERR_UNSUPPORTED.  5 = step-parallel kernel (sweep_sp_kernel.cuh: four lanes per (chain, block), lane s owns step s of every
- * 4-step tile; only the proposal's recursion runs as four rounds with a shuffle broadcast), same conditions, or DMT_ERR_UNSUPPORTED.
- * Automatic: warp-specialised while the grid of (32 chains, block) units fits one round of CTAs, then (models with >= 2 Wiener coordinates)
- * step-parallel up to 14,080 (chain, block) units, then two lanes per (chain, block) in the register-tile kernel while that grid fits one
- * wave, then the pipelined kernel.  Same arithmetic, results equal up to FP64 rounding (different FMA contraction). */
+ * 1 = always the register-tile kernel (fwd_kernel.cuh), with dmt_set_fwd_lanes lanes per (chain, block).  The other kernels need every
+ * chain to own its parameter set in chain order, a uniform law parity and Z == NULL; modes 2, 3 and 5 force one of them and return
+ * DMT_ERR_UNSUPPORTED where these do not hold:
+ *   2 = software-pipelined kernel (sweep_kernel.cuh: guiding term through a TMA shared-memory ring, X double-buffered in registers),
+ *       one lane per (chain, block): DMT_ERR_UNSUPPORTED unless dmt_set_fwd_lanes is 0 or 1;
+ *   3 = warp-specialised kernel (sweep_ws_kernel.cuh: per group of 32 chains and block a CTA of 16 warps that form a pipeline — TMA
+ *       producer, generator warps, inverse solve + accepted likelihood, the proposal's recursion, the proposal's likelihood — over
+ *       shared-memory rings, one CTA per SM);
+ *   5 = step-parallel kernel (sweep_sp_kernel.cuh: four lanes per (chain, block), lane s owns step s of every 4-step tile; only the
+ *       proposal's recursion runs as four rounds with a shuffle broadcast).
+ * 0 (default) = automatic: the register-tile kernel where the conditions above do not hold or dmt_set_fwd_lanes forces lanes; else
+ * warp-specialised while the grid of (32 chains, block) units fits one round of CTAs, then (models with >= 2 Wiener coordinates)
+ * step-parallel up to 14,080 (chain, block) units, then two lanes per (chain, block) in the register-tile kernel while that grid fits
+ * one wave, then the pipelined kernel with lazy noise or the register-tile kernel with eager noise.  Other modes (4 included) are
+ * DMT_ERR_ARG.  Same arithmetic, results equal up to FP64 rounding (different FMA contraction). */
 int32_t dmt_set_sweep_mode(dmt_ctx *ctx, int32_t mode);
-/* Diagnostics: name and thread mapping of the forward kernel (K2-K5) this context launched last, e.g. "sweep_ws_kernel<lazy>",
+/* Diagnostics: name and thread mapping of the forward kernel (K2-K5) this context launched last, e.g. "sweep_ws_kernel<wide, lazy>",
  * "sweep_pipe_kernel<lanes=1, lazy>", "fwd_kernel<op=6, lanes=4>" — what a benchmark should print instead of guessing the automatic
  * choice.  No counterpart in the reference. */
 int32_t dmt_get_last_forward_kernel(dmt_ctx *ctx, char *buf, int32_t len);
