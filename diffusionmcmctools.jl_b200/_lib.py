@@ -94,6 +94,11 @@ SIGNATURES = {
     "dmt_get_last_forward_kernel": (C.c_int32, [_vp, C.c_char_p, C.c_int32]),
     "dmt_get_X_chains": (C.c_int32, [_vp, C.c_int32, C.c_int32, _ip, _dp]),
     "dmt_get_W_chains": (C.c_int32, [_vp, C.c_int32, C.c_int32, _ip, _dp]),
+    "dmt_path_moments_add": (C.c_int32, [_vp]),
+    "dmt_path_moments_reset": (C.c_int32, [_vp]),
+    "dmt_get_path_moments": (C.c_int32, [_vp, C.c_int32, _ip, _dp, _dp, C.POINTER(C.c_uint64)]),
+    "dmt_set_path_moments": (C.c_int32, [_vp, _dp, _dp, C.c_uint64]),
+    "dmt_get_pset_path_moments": (C.c_int32, [_vp, _dp, _dp, _dp]),
     "dmt_get_layout_guiding_term": (C.c_int32, [_vp, C.c_int32, C.c_int32, C.c_int32, _dp, _dp, _dp]),
     "dmt_debug_normals": (C.c_int32, [_vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, _dp]),
     "dmt_debug_exponentials": (C.c_int32, [_vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, _dp]),
@@ -189,6 +194,7 @@ class Ctx:
         rc = self.lib.dmt_create(C.byref(cfg), self.n_pts.ctypes.data_as(_ip), _p(self.tt), pp, C.byref(self.h))
         if rc:
             raise DmtError(rc, (self.lib.dmt_last_error(None) or b"").decode())
+        self.moments_count = 0  # updates in the path-moment accumulators (mirrors the library's count)
         if DEFAULT_FWD_LANES:
             self.set_fwd_lanes(DEFAULT_FWD_LANES)
 
@@ -345,6 +351,36 @@ class Ctx:
         W = np.empty((self.S, self.dw, self.M))
         self._ck(self.lib.dmt_get_W(self.h, side, _p(W)))
         return W
+
+    # -- posterior path moments (per-chain Welford moments of the accepted paths, kept on the device)
+    def path_moments_add(self):
+        """accumulate the current accepted paths of all chains (one kernel launch)"""
+        self._ck(self.lib.dmt_path_moments_add(self.h))
+        self.moments_count += 1
+
+    def path_moments_reset(self):
+        self._ck(self.lib.dmt_path_moments_reset(self.h))
+        self.moments_count = 0
+
+    def get_path_moments(self, chains=None):
+        """-> (mean [NP, d, n], m2 [NP, d, n], count) of the listed chains (None: all M); var = m2 / count"""
+        sel = None if chains is None else np.ascontiguousarray(chains, dtype=np.int32)
+        n = self.M if sel is None else int(sel.size)
+        mean, m2, cnt = np.empty((self.NP, self.d, n)), np.empty((self.NP, self.d, n)), C.c_uint64(0)
+        self._ck(self.lib.dmt_get_path_moments(self.h, n, None if sel is None else sel.ctypes.data_as(_ip), _p(mean), _p(m2), C.byref(cnt)))
+        return mean, m2, int(cnt.value)
+
+    def set_path_moments(self, mean, m2, count):
+        """restore all M chains' moments (as get_path_moments() returned them)"""
+        shape = (self.NP, self.d, self.M)
+        self._ck(self.lib.dmt_set_path_moments(self.h, _p(_f64(mean, shape)), _p(_f64(m2, shape)), int(count)))
+        self.moments_count = int(count)
+
+    def get_pset_path_moments(self):
+        """-> (mean, var, rhat), each [NP, d, P]: pooled over the chains of each parameter / data set (see include/dmt.h)"""
+        out = [np.empty((self.NP, self.d, self.P)) for _ in range(3)]
+        self._ck(self.lib.dmt_get_pset_path_moments(self.h, *(_p(a) for a in out)))
+        return tuple(out)
 
     # -- hot path
     def set_artificial_obs(self, layout):

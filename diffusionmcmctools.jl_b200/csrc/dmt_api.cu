@@ -7,6 +7,7 @@
 #include "sweep_ws_kernel.cuh"
 #include "sweep_sp_kernel.cuh"
 #include "tsit5_kernel.cuh"
+#include "moments_kernel.cuh"
 
 #include <algorithm>
 #include <atomic>
@@ -187,6 +188,11 @@ struct dmt_ctx {
     int G_owner = -1;        // layout whose K1 wrote the shared accepted-law store last (-1: unknown / laws changed)
     bool parP_mixed = false; // a masked swap_PP! made the law parity chain-dependent
     bool aux_all_linearised = true; // every auxiliary law so far came from dmt_set_aux_linearised: B has the Jacobian's sparsity (JacMask)
+    // posterior path moments (dmt_path_moments_add): per-chain Welford accumulators in the X layout, tiles then interval starts,
+    // [NT*D*M*4 + K*D*M] each; allocated on the first update.  Per-pset chain lists (CSR) built on the first pooled read.
+    DevBuf<double> d_pm_mean, d_pm_m2;
+    uint64_t pm_count = 0;
+    DevBuf<int> d_pm_cs, d_pm_chains;
 
     double *scratch(size_t n) {
         if (d_scratch.n < n) d_scratch.alloc(n, false);
@@ -1616,6 +1622,132 @@ int32_t dmt_allreduce_stats(dmt_ctx *ctx, int32_t layout, double *out) {
         if (ctx->nccl_comm) // ONE small allreduce: [sum ll, sum ll°, accept counts per block]  (SURVEY §8e, C1)
             NCK(g_nccl.AllReduce(ctx->d_stats.p, ctx->d_stats.p, (size_t)(2 + L.nb), 8 /* ncclDouble */, 0 /* ncclSum */, ctx->nccl_comm, ctx->stream));
         CK(cudaMemcpyAsync(out, ctx->d_stats.p, sizeof(double) * (2 + L.nb), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    });
+}
+
+} // extern "C"
+
+// ------------------------------------------------------------------------------------------------ posterior path moments
+namespace {
+size_t pm_tile_len(dmt_ctx *c) { return (size_t)c->NT * c->D * c->M * 4; }
+size_t pm_len(dmt_ctx *c) { return pm_tile_len(c) + (size_t)c->K * c->D * c->M; }
+void pm_alloc(dmt_ctx *c) {
+    if (c->d_pm_mean.p) return;
+    const size_t n = pm_len(c);
+    for (DevBuf<double> *b : {&c->d_pm_mean, &c->d_pm_m2}) {
+        if (cudaMalloc(&b->p, n * sizeof(double)) != cudaSuccess) {
+            cudaGetLastError();
+            c->d_pm_mean.release(); c->d_pm_m2.release();
+            throw DmtError(DMT_ERR_CUDA, "path moments: cannot allocate 2 x " + std::to_string(n * sizeof(double)) + " bytes of device memory");
+        }
+        b->n = n;
+    }
+}
+// accumulators <-> natural [NP][d][n] (sel == null: chains 0..n-1)
+void pm_xfer(dmt_ctx *c, double *A, int n, const int32_t *chains, double *host, bool upload) {
+    const size_t len = (size_t)c->NP * c->D * n;
+    DevBuf<double> nat;
+    DevBuf<int> sel;
+    nat.alloc(len, false);
+    if (chains) {
+        sel.alloc(n, false);
+        CK(cudaMemcpyAsync(sel.p, chains, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
+    }
+    if (upload) CK(cudaMemcpyAsync(nat.p, host, len * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    ++g_launches, moments_xfer_kernel<<<dim3((n + 63) / 64, c->K), 64, 0, c->stream>>>(c->dev, c->D, A, A + pm_tile_len(c), sel.p, n, nat.p,
+                                                                                       upload ? 1 : 0);
+    CK(cudaGetLastError());
+    if (!upload) CK(cudaMemcpyAsync(host, nat.p, len * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+}
+template <int D> void launch_path_moments(dmt_ctx *c, double w, int first) {
+    const dim3 grid((unsigned)((c->M + 127) / 128), (unsigned)std::min(c->NT + c->K, 65535), 1);
+    double *mu = c->d_pm_mean.p, *m2 = c->d_pm_m2.p;
+    const size_t t = pm_tile_len(c);
+    ++g_launches, path_moments_kernel<D><<<grid, 128, 0, c->stream>>>(c->dev, mu, m2, mu + t, m2 + t, w, first);
+}
+} // namespace
+
+extern "C" {
+
+int32_t dmt_path_moments_add(dmt_ctx *ctx) {
+    DMT_RANGE("dmt_path_moments_add");
+    return guarded(ctx, [&] {
+        pm_alloc(ctx);
+        const uint64_t n = ctx->pm_count + 1;
+        const double w = 1.0 / (double)n;
+        const int first = n == 1 ? 1 : 0;
+        switch (ctx->D) { // reads X only: under lazy noise W stays as it is
+        case 2: launch_path_moments<2>(ctx, w, first); break;
+        case 3: launch_path_moments<3>(ctx, w, first); break;
+        case 4: launch_path_moments<4>(ctx, w, first); break;
+        case 6: launch_path_moments<6>(ctx, w, first); break;
+        default: throw DmtError(DMT_ERR_UNSUPPORTED, "path moments: no kernel for this state dimension");
+        }
+        CK(cudaGetLastError());
+        ctx->pm_count = n;
+    });
+}
+int32_t dmt_path_moments_reset(dmt_ctx *ctx) {
+    return guarded(ctx, [&] { ctx->pm_count = 0; });
+}
+int32_t dmt_get_path_moments(dmt_ctx *ctx, int32_t n_sel, const int32_t *chains, double *mean, double *m2, uint64_t *count) {
+    return guarded(ctx, [&] {
+        REQUIRE(mean && m2 && count, DMT_ERR_ARG, "null output array");
+        REQUIRE(ctx->pm_count > 0, DMT_ERR_STATE, "no path moments accumulated (dmt_path_moments_add)");
+        if (chains) {
+            REQUIRE(n_sel >= 1, DMT_ERR_ARG, "bad chain selection");
+            for (int i = 0; i < n_sel; i++) REQUIRE(chains[i] >= 0 && chains[i] < ctx->M, DMT_ERR_ARG, "chain index out of range");
+        } else {
+            n_sel = ctx->M;
+        }
+        pm_xfer(ctx, ctx->d_pm_mean.p, n_sel, chains, mean, false);
+        pm_xfer(ctx, ctx->d_pm_m2.p, n_sel, chains, m2, false);
+        *count = ctx->pm_count;
+    });
+}
+int32_t dmt_set_path_moments(dmt_ctx *ctx, const double *mean, const double *m2, uint64_t count) {
+    return guarded(ctx, [&] {
+        REQUIRE(mean && m2, DMT_ERR_ARG, "null input array");
+        REQUIRE(count > 0, DMT_ERR_ARG, "count must be >= 1 (dmt_path_moments_reset clears the moments)");
+        pm_alloc(ctx);
+        pm_xfer(ctx, ctx->d_pm_mean.p, ctx->M, nullptr, (double *)mean, true);
+        pm_xfer(ctx, ctx->d_pm_m2.p, ctx->M, nullptr, (double *)m2, true);
+        ctx->pm_count = count;
+    });
+}
+int32_t dmt_get_pset_path_moments(dmt_ctx *ctx, double *mean, double *var, double *rhat) {
+    return guarded(ctx, [&] {
+        REQUIRE(mean && var && rhat, DMT_ERR_ARG, "null output array");
+        REQUIRE(ctx->pm_count > 0, DMT_ERR_STATE, "no path moments accumulated (dmt_path_moments_add)");
+        const int M = ctx->M, P = ctx->P;
+        if (!ctx->d_pm_cs.p) { // chains of every pset in ascending order
+            std::vector<int> pset(M), cs(P + 1, 0), list(M);
+            CK(cudaMemcpy(pset.data(), ctx->d_pset.p, sizeof(int) * M, cudaMemcpyDeviceToHost));
+            for (int c = 0; c < M; c++) cs[pset[c] + 1]++;
+            for (int q = 0; q < P; q++) cs[q + 1] += cs[q];
+            std::vector<int> fill(cs.begin(), cs.end() - 1);
+            for (int c = 0; c < M; c++) list[fill[pset[c]]++] = c;
+            ctx->d_pm_cs.alloc(P + 1, false);
+            ctx->d_pm_chains.alloc(M, false);
+            CK(cudaMemcpy(ctx->d_pm_cs.p, cs.data(), sizeof(int) * (P + 1), cudaMemcpyHostToDevice));
+            CK(cudaMemcpy(ctx->d_pm_chains.p, list.data(), sizeof(int) * M, cudaMemcpyHostToDevice));
+            CK(cudaStreamSynchronize(cudaStreamLegacy)); // pageable H2D copies return before the DMA lands; ctx->stream does not order against them
+        }
+        const size_t len = (size_t)ctx->NP * ctx->D * P, t = pm_tile_len(ctx);
+        DevBuf<double> out;
+        out.alloc(3 * len, false);
+        int nk_max = 0;
+        for (int k = 0; k < ctx->K; k++) nk_max = std::max(nk_max, ctx->nsteps[k] + 1);
+        const size_t per_k = (size_t)nk_max * ctx->D * P;
+        const double *mu = ctx->d_pm_mean.p, *m2 = ctx->d_pm_m2.p;
+        ++g_launches, pset_moments_kernel<<<dim3((unsigned)((per_k + 127) / 128), ctx->K), 128, 0, ctx->stream>>>(
+            ctx->dev, ctx->D, mu, m2, mu + t, m2 + t, ctx->d_pm_cs.p, ctx->d_pm_chains.p, (double)ctx->pm_count, out.p, out.p + len, out.p + 2 * len);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(mean, out.p, len * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(var, out.p + len, len * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(rhat, out.p + 2 * len, len * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
     });
 }

@@ -130,3 +130,18 @@ def paths(he, side=0):
     """per recording (global order): X [n_points, d] of the accepted (0) or proposal (1) side"""
     per_bucket = [se.ctx.get_X(side) for se in he.buckets]
     return [per_bucket[b][:, :, i] for b, i in (he.where[r] for r in range(he.M_total))]
+
+
+def path_moments_add(he):
+    """add the current accepted paths of every recording to its path moments (host.PathMoments), one launch per bucket"""
+    for se in he.buckets:
+        se.ctx.path_moments_add()
+
+
+def chain_moments(he):
+    """per recording (global order): (mean [n_points, d], var [n_points, d]) of its accepted path, var = m2 / count"""
+    per_bucket = []
+    for se in he.buckets:
+        mean, m2, n = se.ctx.get_path_moments()
+        per_bucket.append((mean, m2 / n))
+    return [(per_bucket[b][0][:, :, i], per_bucket[b][1][:, :, i]) for b, i in (he.where[r] for r in range(he.M_total))]

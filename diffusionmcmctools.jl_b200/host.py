@@ -499,6 +499,41 @@ class PathSaver:
         return [(i, arr) for i, _, arr in self._saved]
 
 
+class PathMoments:
+    """Posterior summary of the accepted paths of EVERY recording, computed where the paths live: the counterpart of PathSaver for
+    the whole ensemble.  Each call at iterations start, start + every, ... adds the current accepted paths to per-recording running
+    moments on the device (one kernel launch, no copy).
+        pm = PathMoments(se, every=10, start=1000);  in the loop: pm(i);  at the end:
+        mean, var = pm.chain_moments()          # [NP, d, M] each: the posterior mean and variance of every recording's path
+        mean, var, rhat = pm.pset_moments()     # [NP, d, P]: pooled over the chains of each data set, with Gelman-Rubin R-hat
+    Point axis as in get_X (concatenated interval grids).  The summaries cover the chains this process holds."""
+
+    def __init__(self, se, every=1, start=0):
+        self.se, self.every, self.start = se, int(every), int(start)
+
+    def __call__(self, mcmciter):
+        if mcmciter < self.start or (mcmciter - self.start) % self.every:
+            return False
+        self.se.ctx.path_moments_add()
+        return True
+
+    @property
+    def count(self):
+        return self.se.ctx.moments_count
+
+    def reset(self):
+        self.se.ctx.path_moments_reset()
+
+    def chain_moments(self, chains=None):
+        """-> (mean, var) [NP, d, n] of the listed recordings (None: all), var = m2 / count (divisor count)"""
+        mean, m2, n = self.se.ctx.get_path_moments(chains)
+        return mean, m2 / n
+
+    def pset_moments(self):
+        """-> (mean, var, rhat) [NP, d, P]; var is the variance of all pooled draws, rhat is NaN where it is undefined"""
+        return self.se.ctx.get_pset_path_moments()
+
+
 class HistoryStreamer:
     """Streams ll_history / accpt_history of a BlockEnsemble to the host in chunks of `every` iterations while the sampler runs
     (b.ll_history, b°.ll_history src/block.jl:57-58; bb.accpt_history src/biblock.jl:47): call it once per iteration AFTER the
@@ -539,8 +574,8 @@ class HistoryStreamer:
 # ---- checkpoint / resume (not in the reference, which keeps its state in Julia objects; SURVEY §5 / §8f item 3) -------------
 def save_state(se, path, layouts=()):
     """Everything needed to continue a run bit-exactly: accepted and proposal X and W (resolved through the parity bits), the
-    accepted and proposal parameters θ / θ°, and per layout the ll fields and the ll / accept histories.  The counter-based
-    generator needs no state beyond (seed, layout, iteration)."""
+    accepted and proposal parameters θ / θ°, per layout the ll fields and the ll / accept histories, and the path moments
+    (PathMoments) when any were accumulated.  The counter-based generator needs no state beyond (seed, layout, iteration)."""
     ctx = se.ctx
     d = dict(X0=ctx.get_X(0), X1=ctx.get_X(1), W0=ctx.get_W(0), W1=ctx.get_W(1), theta=se.theta, theta_o=se.theta_o,
              n_pts=ctx.n_pts, tt=ctx.tt, chain_lo=se.chain_lo, chain_hi=se.chain_hi)
@@ -551,6 +586,8 @@ def save_state(se, path, layouts=()):
             d["acc_hist_%d" % be.layout] = ctx.get_accept_history(be.layout, 0, be.ll_hist_len - 1)
             for s in (0, 1):
                 d["ll_hist%d_%d" % (s, be.layout)] = ctx.get_ll_history(be.layout, s, 0, be.ll_hist_len - 1)
+    if ctx.moments_count > 0:
+        d["moments_mean"], d["moments_m2"], d["moments_count"] = ctx.get_path_moments()
     np.savez_compressed(path, **d)
 
 
@@ -558,12 +595,17 @@ def load_state(se, path, layouts=()):
     """Restore a state written by save_state into an ensemble built with the same recordings, grids, seed and layouts.
     The laws are restored too: θ / θ° go back to the device (through the law parity, so it does not matter how many
     swap_PP! the saved run had made), the Jacobian-linearised auxiliary laws are re-evaluated at the stored points, and the guiding
-    term of every layout in `layouts` is recomputed (in order; layouts sharing the store are recomputed by the sweep loop anyway)."""
+    term of every layout in `layouts` is recomputed (in order; layouts sharing the store are recomputed by the sweep loop anyway).
+    Path moments are restored when the checkpoint has them and reset when it has none."""
     z = np.load(path)
     ctx = se.ctx
     if not (np.array_equal(z["n_pts"], ctx.n_pts) and np.array_equal(z["tt"], ctx.tt) and int(z["chain_lo"]) == se.chain_lo and int(z["chain_hi"]) == se.chain_hi):
         raise ValueError("checkpoint belongs to a different ensemble (grid or chain slice differ)")
     ctx.set_X(z["X0"], 0); ctx.set_X(z["X1"], 1); ctx.set_W(z["W0"], 0); ctx.set_W(z["W1"], 1)
+    if "moments_count" in z:
+        ctx.set_path_moments(z["moments_mean"], z["moments_m2"], int(z["moments_count"]))
+    else:
+        ctx.path_moments_reset()
     se.theta, se.theta_o = z["theta"].copy(), z["theta_o"].copy()
     sides = ((0, se.theta), (1, se.theta_o)) if se.two_sided else ((0, se.theta),)
     for side, th in sides:

@@ -137,6 +137,34 @@ int32_t dmt_get_W(dmt_ctx *ctx, int32_t side, double *W);
 int32_t dmt_get_X_chains(dmt_ctx *ctx, int32_t side, int32_t n_sel, const int32_t *chains, double *X);
 int32_t dmt_get_W_chains(dmt_ctx *ctx, int32_t side, int32_t n_sel, const int32_t *chains, double *W);
 
+/* ---- posterior summaries of the paths ------------------------------------------------------------------------- */
+/* The smoothing tutorials keep a copy of the accepted path every few hundred iterations (docs/src/tutorials/biblock/smoothing.md:55)
+ * and summarise the copies by their mean and spread.  Here every chain carries running moments of its ACCEPTED path on the device
+ * instead: Welford updates, one streaming launch over X per call, no copy of the paths.  Point axis as in dmt_get_X (concatenated
+ * per-interval grids, boundary points twice).  Memory: 16 d (S + K) M bytes (mean and m2), allocated by the first update (or set),
+ * freed by dmt_destroy; failing allocation is DMT_ERR_CUDA.  The update reads X only (under lazy noise W is not rebuilt).
+ * The moments describe the chains THIS context holds: per-chain moments are keyed by the chain, so a sharded run has exactly the
+ * unsharded per-chain moments; the pooled moments below cover this rank's chains only. */
+/* accumulate the current accepted paths of all chains (the `deepcopy(bb.b.XX)` step of docs/src/tutorials/biblock/smoothing.md:55);
+ * count := count + 1.  n = count: mean += (x - mean) / n, m2 += (x - mean_old)(x - mean_new), each operation rounded on its own */
+int32_t dmt_path_moments_add(dmt_ctx *ctx);
+/* count := 0; the buffers are kept (the next update starts afresh) — e.g. at the end of burn-in */
+int32_t dmt_path_moments_reset(dmt_ctx *ctx);
+/* mean[NP][d][n_sel], m2[NP][d][n_sel] (sum of squared deviations: var = m2 / count) of the listed chains (chains == NULL: all M,
+ * n_sel ignored); *count = number of updates.  DMT_ERR_STATE when count == 0, DMT_ERR_ARG for a chain index out of range.
+ * The posterior mean and band of every recording of docs/src/tutorials/biblock/smoothing.md:55 without copying paths. */
+int32_t dmt_get_path_moments(dmt_ctx *ctx, int32_t n_sel, const int32_t *chains, double *mean, double *m2, uint64_t *count);
+/* restore all M chains' moments as dmt_get_path_moments(chains = NULL) returned them (checkpoint / resume of the saving loop of
+ * docs/src/tutorials/biblock/smoothing.md:55); count == 0 is DMT_ERR_ARG (use dmt_path_moments_reset) */
+int32_t dmt_set_path_moments(dmt_ctx *ctx, const double *mean, const double *m2, uint64_t count);
+/* pooled over the chains that share a parameter / data set (chains c with pset_of_chain[c] == q, m of them), [NP][d][P]:
+ *   mean = (1/m) sum mu_c;  var = (sum m2_c / n + sum (mu_c - mean)^2) / m, the variance of all n m draws;
+ *   rhat = sqrt(var+ / W), the Gelman-Rubin statistic with W = sum m2_c / (m (n-1)), B = n sum (mu_c - mean)^2 / (m-1),
+ *   var+ = (n-1)/n W + B/n; NaN when m < 2, n < 2 or W == 0 (e.g. at the known start point).
+ * Sums in a fixed order: bitwise reproducible for a given (M, pset map).  LOCAL to this context (rank): pooling across GPUs is
+ * not done here.  The ensemble-wide summary of many chains on one recording (docs/src/tutorials/biblock/smoothing.md:55). */
+int32_t dmt_get_pset_path_moments(dmt_ctx *ctx, double *mean, double *var, double *rhat);
+
 /* ---- the hot path --------------------------------------------------------------------------------------------- */
 /* GP.set_obs!(be)                          src/block_ensemble.jl:192 -> src/biblock.jl:275-280            (K7) */
 int32_t dmt_set_artificial_obs(dmt_ctx *ctx, int32_t layout);

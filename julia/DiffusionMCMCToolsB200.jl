@@ -415,6 +415,29 @@ histories_async!(ll::Array{Float64,4}, acc::Array{UInt8,3}, be::DBE, range) =   
                            be.se.ctx, be.layout, first(range) - 1, last(range) - 1, ll, acc))
 snapshot_wait(se::DeviceEnsemble) = check(se.ctx, ccall((:dmt_snapshot_wait, libdmt), Int32, (Ptr{Cvoid},), se.ctx))
 
+# ---- posterior summaries of the paths: per-recording running moments of the accepted path, on the device (include/dmt.h) -------
+# The tutorials' `paths[i ÷ 400] = deepcopy(bb.b.XX)` (docs/src/tutorials/biblock/smoothing.md:55) summarised by mean and variance for
+# every recording, without copying paths: call `path_moments_add!(se)` at each saving iteration, read the summaries at the end.
+path_moments_add!(se::DeviceEnsemble) = check(se.ctx, ccall((:dmt_path_moments_add, libdmt), Int32, (Ptr{Cvoid},), se.ctx))
+path_moments_reset!(se::DeviceEnsemble) = check(se.ctx, ccall((:dmt_path_moments_reset, libdmt), Int32, (Ptr{Cvoid},), se.ctx))
+"""    path_moments(se, recs=1:se.M) -> (mean, var, count): mean and var of size (length(recs), d, NP), var = m2 / count"""
+function path_moments(se::DeviceEnsemble, recs::AbstractVector{<:Integer}=1:se.M)
+    sel = Int32.(recs .- 1)
+    mean = Array{Float64,3}(undef, length(sel), se.d, sum(se.n_pts)); m2 = similar(mean); n = Ref{UInt64}(0)
+    check(se.ctx, ccall((:dmt_get_path_moments, libdmt), Int32, (Ptr{Cvoid}, Int32, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ref{UInt64}),
+                        se.ctx, length(sel), sel, mean, m2, n))
+    mean, m2 ./ n[], Int(n[])
+end
+"""restore all recordings' moments from `mean`, `m2` (size (M, d, NP)) after `count` updates (checkpoint / resume)"""
+set_path_moments!(se::DeviceEnsemble, mean::Array{Float64,3}, m2::Array{Float64,3}, count::Integer) =
+    check(se.ctx, ccall((:dmt_set_path_moments, libdmt), Int32, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, UInt64), se.ctx, mean, m2, count))
+"""    pset_path_moments(se) -> (mean, var, rhat), each (P, d, NP): pooled over the recordings that share a data set; Gelman-Rubin R-hat"""
+function pset_path_moments(se::DeviceEnsemble)
+    mean = Array{Float64,3}(undef, se.P, se.d, sum(se.n_pts)); var = similar(mean); rhat = similar(mean)
+    check(se.ctx, ccall((:dmt_get_pset_path_moments, libdmt), Int32, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}), se.ctx, mean, var, rhat))
+    mean, var, rhat
+end
+
 # ---- BlockCollection / BiBlock views (src/block_collection.jl:17-36, src/biblock.jl:17-62) ---------------------------------
 # `be.recordings[r]` and `.blocks[b]` of the reference.  The numerical calls are batched over all recordings and blocks on the device —
 # call them on the DeviceBlockEnsemble; the views carry what acts on ONE recording / ONE block: reading XX, WW, ll and the histories,
@@ -474,6 +497,7 @@ ll_of_accepted(bb::DeviceBiBlock, i::Integer) = ll_of_accepted(bb.be, i)[bb.rec,
 ll_of_accepted(bc::DeviceBlockCollection, i::Integer) = ll_of_accepted(bc.be, i)[bc.rec, :]                       # src/block_collection.jl:172
 
 export DeviceEnsemble, DeviceBlockEnsemble, DeviceBlockCollection, DeviceBiBlock, upload_aux!, get_paths, get_X, get_W, trajectories,
-    wiener_trajectories, pack_paths, pack_noise, recordings, blocks, blocking_sweep!, enable_guiding_cache!
+    wiener_trajectories, pack_paths, pack_noise, recordings, blocks, blocking_sweep!, enable_guiding_cache!, path_moments_add!,
+    path_moments_reset!, path_moments, set_path_moments!, pset_path_moments
 
 end # module
