@@ -105,6 +105,10 @@ struct Layout {
     bool F_stale = false; // cache valid but F/c of the private store not materialised for the current artificial observations
     DevBuf<double> d_Gl[2], d_c0l[2], d_FP[2], d_cq, d_vlast;
     DevBuf<int> d_blk_of_k;
+    // the persistent schedule of the pipelined sweep (PipeSched, sweep_kernel.cuh): its task entries, tickets and hand-over state
+    DevBuf<int> d_task;
+    DevBuf<unsigned> d_ticket;
+    DevBuf<double> d_hand;
 };
 
 // ---- NCCL, resolved at run time so that libdmt.so has no link-time dependency on it
@@ -182,6 +186,7 @@ struct dmt_ctx {
     int sweep_mode = 0;      // dmt_set_sweep_mode: 0 = automatic (pick_sweep), 1 = register-tile kernel, 2 / 3 / 5 = pipelined /
                              // warp-specialised / step-parallel kernel or error
     std::unordered_map<const void *, size_t> resident; // kernel -> CTAs resident at once on this context's device (resident_ctas)
+    int n_sm = 0;            // SMs of this context's device (resident_ctas)
     bool lazy_W = false;     // dmt_set_lazy_noise: blocking sweeps do not materialise W_acc / W°
     char last_fwd_kernel[96] = ""; // name and mapping of the forward kernel launched last (dmt_get_last_forward_kernel)
     int W_stale_layout = -1; // >= 0: W_acc is not materialised; K5 over this layout rebuilds it (ensure_W)
@@ -226,11 +231,11 @@ dim3 pset_grid(dmt_ctx *c, int ny, int tpb, int nz = 1) { return dim3((c->P + tp
 template <class Kernel> size_t resident_ctas(dmt_ctx *c, Kernel *kernel, int threads, size_t smem) {
     const auto it = c->resident.find((const void *)kernel);
     if (it != c->resident.end()) return it->second;
-    int per_sm = 0, sms = 0;
+    int per_sm = 0;
     CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
-    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
-    return c->resident[(const void *)kernel] = (size_t)per_sm * sms;
+    if (!c->n_sm) CK(cudaDeviceGetAttribute(&c->n_sm, cudaDevAttrMultiProcessorCount, c->cfg.device));
+    return c->resident[(const void *)kernel] = (size_t)per_sm * c->n_sm;
 }
 
 // ---- the register-tile kernel (fwd_kernel.cuh): G lanes per (chain, block), G > 1 for the ops that draw normals
@@ -286,13 +291,31 @@ bool covers_all_intervals(dmt_ctx *c, const Layout &L) {
 
 // ---- the other kernels of the fused sweep pass.  All three need one parameter set per chain in chain order, uniform law parity
 // and device RNG; each is compiled with and without lazy noise.
-// the software-pipelined sweep (sweep_kernel.cuh): one lane per (chain, block), guiding term through a TMA shared-memory ring
+// the software-pipelined sweep (sweep_kernel.cuh): one lane per (chain, block), guiding term through a TMA shared-memory ring.
+// Schedule, with S = 4 schedulers x SMs and U = (32-chain group, block) units: one unit per warp leaves up to three warps on some
+// schedulers, and the pass lasts as long as those do (Lorenz, C3: 1.40 / 1.72 / 2.32 ms for at most 1 / 2 / 3 warps per scheduler,
+// profiles/r02_tuning.md §4d).  So where U allows an even spread the grid is persistent (PipeSched) and warps take the units'
+// intervals by ticket: 2S warps, two on every scheduler, when U >= 2S; S warps when S <= U < 1.23 S (1.23 = 1.72 / 1.40: one warp per
+// scheduler at the one-warp rate beats U / S warps at the two-warp rate); else one unit per warp.  For d <= 3 the warps come four to a
+// CTA, two CTAs per SM; wider models keep one-warp CTAs (four warps' rings do not fit twice).  profiles/r03_tuning.md.
 template <class MD, bool LAZY> void launch_sweep_pipe(dmt_ctx *c, Layout &L, const FwdArgs &fa) {
     constexpr size_t smem = sweep_pipe_smem<MD>();
-    resident_ctas(c, sweep_pipe_kernel<MD, LAZY>, 32, smem);
-    const dim3 grid((unsigned)((c->M + 31) / 32), L.nb, 1);
+    constexpr int WPC = MD::D <= 3 ? 4 : 1;
+    const size_t groups = (c->M + 31) / 32, units = groups * L.nb;
+    const size_t warps = resident_ctas(c, sweep_pipe_kernel<MD, LAZY, WPC>, 32 * WPC, WPC * smem) * WPC;
+    const size_t S = (size_t)c->n_sm * 4;
+    const size_t n = std::min(warps, units >= 2 * S ? 2 * S : (units >= S && units * 100 < S * 123) ? S : 0);
     snprintf(c->last_fwd_kernel, sizeof(c->last_fwd_kernel), "sweep_pipe_kernel<lanes=1%s>", LAZY ? ", lazy" : "");
-    ++g_launches, sweep_pipe_kernel<MD, LAZY><<<grid, 32, smem, c->stream>>>(c->dev, L.dev, fa);
+    if (n < S) {
+        resident_ctas(c, sweep_pipe_kernel<MD, LAZY, 1>, 32, smem);
+        ++g_launches, sweep_pipe_kernel<MD, LAZY, 1><<<dim3((unsigned)groups, L.nb, 1), 32, smem, c->stream>>>(c->dev, L.dev, fa, PipeSched{});
+        return;
+    }
+    if (L.d_ticket.n != 1 + units) L.d_ticket.alloc(1 + units, false);
+    if (L.d_hand.n != (size_t)(MD::D + 3) * units * 32) L.d_hand.alloc((size_t)(MD::D + 3) * units * 32, false);
+    CK(cudaMemsetAsync(L.d_ticket.p, 0, sizeof(unsigned) * (1 + units), c->stream));
+    const PipeSched sc{L.d_task.p, (int)(L.d_task.n * groups), L.d_ticket.p, L.d_hand.p};
+    ++g_launches, sweep_pipe_kernel<MD, LAZY, WPC><<<(unsigned)(n / WPC), 32 * WPC, WPC * smem, c->stream>>>(c->dev, L.dev, fa, sc);
 }
 // the warp-specialised sweep (sweep_ws_kernel.cuh): a pipeline of 16 warps per group of 32 chains and block, one CTA per SM.  Six
 // generator warps; ring depths by state dimension (a stage of the G ring is (d(d+1)/2 + d) KiB, the D ring holds the same again per
@@ -976,6 +999,17 @@ int32_t dmt_set_blocks(dmt_ctx *ctx, int32_t layout, int32_t n_blocks, const int
         L.dev.i0 = L.d_i0.p; L.dev.i1 = L.d_i1.p; L.dev.last = L.d_last.p; L.dev.rho = L.d_rho.p;
         L.dev.ll = L.d_ll.p; L.dev.ok = L.d_ok.p; L.dev.last_acc = L.d_last_acc.p;
         L.dev.acc_hist = hl ? L.d_acc_hist.p : nullptr; L.dev.ll_hist = hl ? L.d_ll_hist.p : nullptr; L.dev.hist_len = (int)hl;
+        {   // the pipelined sweep's task entries (PipeSched): (block b, its interval j) as b + 64 j, every block's first interval first
+            std::vector<int> task;
+            for (int j = 0;; j++) {
+                const size_t n0 = task.size();
+                for (int b = 0; b < n_blocks; b++)
+                    if (i0[b] + j <= i1[b]) task.push_back(b + 64 * j);
+                if (task.size() == n0) break;
+            }
+            L.d_task.alloc(task.size(), false);
+            CK(cudaMemcpy(L.d_task.p, task.data(), sizeof(int) * task.size(), cudaMemcpyHostToDevice));
+        }
         L.set = true;
         L.cache_enabled = false; L.cache_valid = false;
         cache_set_private(L, false);
