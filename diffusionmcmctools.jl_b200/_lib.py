@@ -54,6 +54,12 @@ SIGNATURES = {
     "dmt_equalize_laws": (C.c_int32, [_vp, C.c_int32, C.c_int32, C.c_int32, _ip]),
     "dmt_set_blocks": (C.c_int32, [_vp, C.c_int32, C.c_int32, _ip, _ip, _dp, _bp, C.c_int32]),
     "dmt_set_rho": (C.c_int32, [_vp, C.c_int32, _dp]),
+    "dmt_set_rho_chains": (C.c_int32, [_vp, C.c_int32, _dp]),
+    "dmt_get_rho_chains": (C.c_int32, [_vp, C.c_int32, _dp]),
+    "dmt_set_rho_adaptation": (C.c_int32, [_vp, C.c_int32, C.c_double, C.c_double, C.c_double, C.c_int32, C.c_double, C.c_double]),
+    "dmt_adapt_rho": (C.c_int32, [_vp, C.c_int32]),
+    "dmt_get_rho_adaptation_state": (C.c_int32, [_vp, C.c_int32, _dp, _ip, C.POINTER(C.c_uint64)]),
+    "dmt_set_rho_adaptation_state": (C.c_int32, [_vp, C.c_int32, _dp, _ip, C.c_uint64]),
     "dmt_set_start": (C.c_int32, [_vp, _dp]),
     "dmt_init_paths": (C.c_int32, [_vp, C.c_int32, C.c_uint32, C.c_int32, _ip]),
     "dmt_set_X": (C.c_int32, [_vp, C.c_int32, _dp]),
@@ -289,6 +295,39 @@ class Ctx:
     def set_rho(self, layout, rho):
         rho = _f64(np.broadcast_to(np.asarray(rho, dtype=np.float64), (self.layout_nb[layout],)))
         self._ck(self.lib.dmt_set_rho(self.h, layout, _p(rho)))
+
+    def set_rho_chains(self, layout, rho):
+        """ρ of every (block, chain): anything that broadcasts to [n_blocks, M]"""
+        shape = (self.layout_nb[layout], self.M)
+        rho = _f64(np.broadcast_to(np.asarray(rho, dtype=np.float64), shape), shape)
+        self._ck(self.lib.dmt_set_rho_chains(self.h, layout, _p(rho)))
+
+    def get_rho_chains(self, layout):
+        rho = np.empty((self.layout_nb[layout], self.M))
+        self._ck(self.lib.dmt_get_rho_chains(self.h, layout, _p(rho)))
+        return rho
+
+    def set_rho_adaptation(self, layout, target, gamma0=1.0, decay=0.66, window=10, rho_min=0.0, rho_max=0.999):
+        """target <= 0: freeze ρ (adaptation off); see include/dmt.h for the rule"""
+        self._ck(self.lib.dmt_set_rho_adaptation(self.h, layout, float(target), float(gamma0), float(decay), int(window),
+                                                 float(rho_min), float(rho_max)))
+
+    def adapt_rho(self, layout):
+        self._ck(self.lib.dmt_adapt_rho(self.h, layout))
+
+    def get_rho_adaptation_state(self, layout):
+        """-> (s [n_blocks, M], nacc [n_blocks, M] int32, calls)"""
+        shape = (self.layout_nb[layout], self.M)
+        s, nacc, calls = np.empty(shape), np.empty(shape, dtype=np.int32), C.c_uint64(0)
+        self._ck(self.lib.dmt_get_rho_adaptation_state(self.h, layout, _p(s), nacc.ctypes.data_as(_ip), C.byref(calls)))
+        return s, nacc, int(calls.value)
+
+    def set_rho_adaptation_state(self, layout, s, nacc, calls):
+        shape = (self.layout_nb[layout], self.M)
+        s = _f64(s, shape)
+        nacc = np.ascontiguousarray(nacc, dtype=np.int32)
+        assert nacc.shape == shape
+        self._ck(self.lib.dmt_set_rho_adaptation_state(self.h, layout, _p(s), nacc.ctypes.data_as(_ip), int(calls)))
 
     # -- paths
     def set_start(self, x0):

@@ -98,8 +98,16 @@ struct Layout {
     std::vector<uint8_t> last;
     DevBuf<int> d_i0, d_i1;
     DevBuf<uint8_t> d_last, d_ok, d_last_acc, d_acc_hist;
-    DevBuf<double> d_rho, d_ll, d_ll_hist;
+    DevBuf<double> d_rho, d_ll, d_ll_hist; // d_rho: [nb][M]
     LayoutDev dev{};
+    // pCN memory adaptation (dmt_set_rho_adaptation): per (block, chain) the logit s of ρ in (rho_min, rho_max) and the accepts of the
+    // current window; the call counter is the same on every rank, so it stays on the host
+    bool adapt = false;
+    double ad_target = 0, ad_gamma0 = 0, ad_decay = 0, ad_rho_min = 0, ad_rho_max = 0;
+    int ad_window = 0;
+    uint64_t ad_calls = 0;
+    DevBuf<double> d_ad_s;
+    DevBuf<int32_t> d_ad_nacc;
     // guiding cache (dmt_enable_guiding_cache): layout-private accepted-law guiding term + its affine decomposition in v
     bool cache_enabled = false, cache_valid = false;
     bool F_stale = false; // cache valid but F/c of the private store not materialised for the current artificial observations
@@ -660,6 +668,29 @@ void fill_stats(dmt_ctx *c, Layout &L, double *host_out /* [2+3nb] */) {
     }
 }
 
+// ---- ρ per (block, chain): rho[b] of every chain, [nb][M]
+std::vector<double> rho_per_chain(dmt_ctx *c, int nb, const double *rho) {
+    std::vector<double> r((size_t)nb * c->M);
+    for (int b = 0; b < nb; b++) std::fill(r.begin() + (size_t)b * c->M, r.begin() + (size_t)(b + 1) * c->M, rho[b]);
+    return r;
+}
+// adaptation (re)starts from ρ: s = logit of ρ's position in (rho_min, rho_max), kept 1e-6 away from either end; nacc = 0
+void restart_adaptation(dmt_ctx *c, Layout &L, const std::vector<double> &rho) {
+    std::vector<double> s(rho.size());
+    for (size_t i = 0; i < rho.size(); i++) {
+        const double u = std::min(std::max((rho[i] - L.ad_rho_min) / (L.ad_rho_max - L.ad_rho_min), 1e-6), 1.0 - 1e-6);
+        s[i] = std::log(u / (1.0 - u));
+    }
+    CK(cudaMemcpyAsync(L.d_ad_s.p, s.data(), sizeof(double) * s.size(), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemsetAsync(L.d_ad_nacc.p, 0, sizeof(int32_t) * L.d_ad_nacc.n, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+}
+void upload_rho(dmt_ctx *c, Layout &L, const std::vector<double> &rho) {
+    CK(cudaMemcpyAsync(L.d_rho.p, rho.data(), sizeof(double) * rho.size(), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    if (L.adapt) restart_adaptation(c, L, rho);
+}
+
 // NVTX range around a C-ABI operation (nsys / ncu --nvtx): off unless DMT_NVTX=1, so the hot loop pays one predictable branch
 struct NvtxRange {
     bool on;
@@ -982,12 +1013,17 @@ int32_t dmt_set_blocks(dmt_ctx *ctx, int32_t layout, int32_t n_blocks, const int
         const size_t M = ctx->M;
         L.nb = n_blocks;
         L.i0.assign(i0, i0 + n_blocks); L.i1.assign(i1, i1 + n_blocks); L.last = lst;
-        L.d_i0.alloc(n_blocks); L.d_i1.alloc(n_blocks); L.d_last.alloc(n_blocks); L.d_rho.alloc(n_blocks);
+        L.d_i0.alloc(n_blocks); L.d_i1.alloc(n_blocks); L.d_last.alloc(n_blocks); L.d_rho.alloc(n_blocks * M);
         L.d_ll.alloc(2 * n_blocks * M); L.d_ok.alloc(n_blocks * M); L.d_last_acc.alloc(n_blocks * M);
         CK(cudaMemcpy(L.d_i0.p, i0, sizeof(int) * n_blocks, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(L.d_i1.p, i1, sizeof(int) * n_blocks, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(L.d_last.p, lst.data(), n_blocks, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(L.d_rho.p, rho, sizeof(double) * n_blocks, cudaMemcpyHostToDevice));
+        {
+            const std::vector<double> rr = rho_per_chain(ctx, n_blocks, rho);
+            CK(cudaMemcpy(L.d_rho.p, rr.data(), sizeof(double) * rr.size(), cudaMemcpyHostToDevice));
+        }
+        L.adapt = false;
+        L.d_ad_s.release(); L.d_ad_nacc.release();
         {   // Block ctor: ll = -Inf (src/block.jl:74)
             std::vector<double> ninf(2 * n_blocks * M, -INFINITY);
             CK(cudaMemcpy(L.d_ll.p, ninf.data(), sizeof(double) * ninf.size(), cudaMemcpyHostToDevice));
@@ -1021,8 +1057,93 @@ int32_t dmt_set_rho(dmt_ctx *ctx, int32_t layout, const double *rho) {
     return guarded(ctx, [&] {
         Layout &L = layout_of(ctx, layout);
         REQUIRE(rho, DMT_ERR_ARG, "null rho");
-        CK(cudaMemcpyAsync(L.d_rho.p, rho, sizeof(double) * L.nb, cudaMemcpyHostToDevice, ctx->stream));
+        for (int b = 0; b < L.nb; b++) REQUIRE(std::abs(rho[b]) <= 1.0, DMT_ERR_ARG, "rho must be in [-1, 1]");
+        upload_rho(ctx, L, rho_per_chain(ctx, L.nb, rho));
+    });
+}
+int32_t dmt_set_rho_chains(dmt_ctx *ctx, int32_t layout, const double *rho) {
+    return guarded(ctx, [&] {
+        Layout &L = layout_of(ctx, layout);
+        REQUIRE(rho, DMT_ERR_ARG, "null rho");
+        const size_t n = (size_t)L.nb * ctx->M;
+        for (size_t i = 0; i < n; i++) REQUIRE(std::abs(rho[i]) <= 1.0, DMT_ERR_ARG, "rho must be in [-1, 1]");
+        upload_rho(ctx, L, std::vector<double>(rho, rho + n));
+    });
+}
+int32_t dmt_get_rho_chains(dmt_ctx *ctx, int32_t layout, double *out) {
+    return guarded(ctx, [&] {
+        Layout &L = layout_of(ctx, layout);
+        REQUIRE(out, DMT_ERR_ARG, "null");
+        CK(cudaMemcpyAsync(out, L.d_rho.p, sizeof(double) * L.d_rho.n, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
+    });
+}
+int32_t dmt_set_rho_adaptation(dmt_ctx *ctx, int32_t layout, double target, double gamma0, double decay, int32_t window, double rho_min,
+                               double rho_max) {
+    return guarded(ctx, [&] {
+        Layout &L = layout_of(ctx, layout);
+        if (!(target > 0.0)) { // (NaN included: nothing to adapt toward)
+            REQUIRE(!std::isnan(target), DMT_ERR_ARG, "target is NaN");
+            L.adapt = false;
+            L.d_ad_s.release(); L.d_ad_nacc.release();
+            return;
+        }
+        REQUIRE(target < 1.0 && gamma0 > 0.0 && std::isfinite(gamma0) && decay > 0.5 && decay <= 1.0 && window >= 1, DMT_ERR_ARG,
+                "need 0 < target < 1, gamma0 > 0, 0.5 < decay <= 1 and window >= 1");
+        REQUIRE(rho_min >= 0.0 && rho_min < rho_max && rho_max <= 1.0, DMT_ERR_ARG, "need 0 <= rho_min < rho_max <= 1");
+        L.ad_target = target; L.ad_gamma0 = gamma0; L.ad_decay = decay; L.ad_window = window;
+        L.ad_rho_min = rho_min; L.ad_rho_max = rho_max;
+        const size_t n = (size_t)L.nb * ctx->M;
+        if (L.d_ad_s.n != n) { L.d_ad_s.alloc(n, false); L.d_ad_nacc.alloc(n, false); }
+        std::vector<double> rho(n);
+        CK(cudaMemcpyAsync(rho.data(), L.d_rho.p, sizeof(double) * n, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        L.adapt = true;
+        L.ad_calls = 0;
+        restart_adaptation(ctx, L, rho);
+    });
+}
+int32_t dmt_adapt_rho(dmt_ctx *ctx, int32_t layout) {
+    DMT_RANGE("dmt_adapt_rho");
+    return guarded(ctx, [&] {
+        Layout &L = layout_of(ctx, layout);
+        REQUIRE(L.adapt, DMT_ERR_ARG, "rho adaptation is off for this layout (dmt_set_rho_adaptation)");
+        const uint64_t calls = L.ad_calls + 1;
+        const bool update = calls % (uint64_t)L.ad_window == 0;
+        const double gamma = update ? L.ad_gamma0 * std::pow((double)(calls / (uint64_t)L.ad_window), -L.ad_decay) : 0.0;
+        const int n = L.nb * ctx->M;
+        ++g_launches, adapt_rho_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(L.d_rho.p, L.d_ad_s.p, L.d_ad_nacc.p, L.d_last_acc.p, n,
+                                                                              L.ad_window, update ? 1 : 0, gamma, L.ad_target,
+                                                                              L.ad_rho_min, L.ad_rho_max);
+        CK(cudaGetLastError());
+        L.ad_calls = calls;
+    });
+}
+int32_t dmt_get_rho_adaptation_state(dmt_ctx *ctx, int32_t layout, double *s, int32_t *nacc, uint64_t *calls) {
+    return guarded(ctx, [&] {
+        Layout &L = layout_of(ctx, layout);
+        REQUIRE(L.adapt, DMT_ERR_STATE, "rho adaptation is off for this layout (dmt_set_rho_adaptation)");
+        REQUIRE(s && nacc && calls, DMT_ERR_ARG, "null output");
+        CK(cudaMemcpyAsync(s, L.d_ad_s.p, sizeof(double) * L.d_ad_s.n, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(nacc, L.d_ad_nacc.p, sizeof(int32_t) * L.d_ad_nacc.n, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        *calls = L.ad_calls;
+    });
+}
+int32_t dmt_set_rho_adaptation_state(dmt_ctx *ctx, int32_t layout, const double *s, const int32_t *nacc, uint64_t calls) {
+    return guarded(ctx, [&] {
+        Layout &L = layout_of(ctx, layout);
+        REQUIRE(L.adapt, DMT_ERR_STATE, "rho adaptation is off for this layout (dmt_set_rho_adaptation)");
+        REQUIRE(s && nacc, DMT_ERR_ARG, "null input");
+        const size_t n = (size_t)L.nb * ctx->M;
+        for (size_t i = 0; i < n; i++) {
+            REQUIRE(std::isfinite(s[i]), DMT_ERR_ARG, "s must be finite");
+            REQUIRE(nacc[i] >= 0 && nacc[i] < L.ad_window, DMT_ERR_ARG, "need 0 <= nacc < window");
+        }
+        CK(cudaMemcpyAsync(L.d_ad_s.p, s, sizeof(double) * n, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(L.d_ad_nacc.p, nacc, sizeof(int32_t) * n, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        L.ad_calls = calls;
     });
 }
 

@@ -103,7 +103,7 @@ __global__ void __launch_bounds__(TPB, fwd_minb<MD, G>()) fwd_kernel(const DevCt
     const int win_side = (OP == OP_RECOMPUTE) ? fa.w_side : 0;
     const int wout_side = (OP == OP_DRAW) ? 1 : 0; // SWEEP writes both: accepted in place, proposal to the other buffer
     const int ll_side = (OP == OP_DRAW) ? 1 : law_side;
-    const double rho = (OP == OP_DRAW || SWEEP) ? ly.rho[b] : 0.0;
+    const double rho = (OP == OP_DRAW || SWEEP) ? layout_rho(ly, b, c, M) : 0.0;
     const double crho = (OP == OP_DRAW || SWEEP) ? sqrt(1.0 - rho * rho) : 1.0;
     const int skip = fa.skip;
     const size_t gstr = P * 4; // doubles between components of one tile

@@ -65,7 +65,7 @@ struct LayoutDev {
     int nb, id;
     const int *i0, *i1;
     const uint8_t *last;
-    const double *rho;
+    const double *rho; // [nb][M] pCN memory of every (block, chain), bb.ρ (src/biblock.jl:46): read through layout_rho only
     double *ll;        // [2][nb][M]
     uint8_t *ok;       // [nb][M] success of the last forward op
     uint8_t *last_acc; // [nb][M]
@@ -87,6 +87,9 @@ struct BwdArgs {
     int use_override; // 1: every non-terminal block uses v[] as its artificial observation (cache build probes)
     double v[6];
 };
+
+// ρ of block b for the context's local chain c (M = the context's chain count): the one place that knows how LayoutDev::rho is laid out
+__device__ __forceinline__ double layout_rho(const LayoutDev &ly, int b, int c, size_t M) { return ly.rho[(size_t)b * M + c]; }
 
 enum { OP_DRAW = 0, OP_RECOMPUTE = 1, OP_LOGLIK = 2, OP_INVSOLVE = 3, OP_INVSOLVE_LL = 4, OP_INIT = 5, OP_SWEEP = 6 };
 
@@ -971,6 +974,23 @@ __global__ void accept_kernel(const DevCtx cx, const LayoutDev ly, uint32_t iter
         ly.ll_hist[((size_t)iter * 2 + 1) * ly.nb * M + idx] = llo;
     }
     if (acc) { ly.ll[idx] = llo; ly.ll[(size_t)ly.nb * M + idx] = ll; }
+}
+
+// dmt_adapt_rho: one thread per (block, chain).  nacc += the last accept decision; at the end of a window (update != 0) the logit s of
+// ρ in (rho_min, rho_max) moves by gamma (target - nacc / window) and nacc restarts.  The update is rounded step by step, without
+// FMA contraction, so that a host restatement in IEEE double reproduces s exactly.  Low acceptance raises ρ: smaller moves.
+__global__ void adapt_rho_kernel(double *rho, double *s, int32_t *nacc, const uint8_t *last_acc, int n, int window, int update,
+                                 double gamma, double target, double rho_min, double rho_max) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int32_t a = nacc[i] + (last_acc[i] ? 1 : 0);
+    if (update) {
+        const double si = __dadd_rn(s[i], __dmul_rn(gamma, __dsub_rn(target, __ddiv_rn((double)a, (double)window))));
+        s[i] = si;
+        rho[i] = __dadd_rn(rho_min, __ddiv_rn(__dsub_rn(rho_max, rho_min), __dadd_rn(1.0, exp(-si))));
+        a = 0;
+    }
+    nacc[i] = a;
 }
 
 __global__ void save_ll_kernel(const DevCtx cx, const LayoutDev ly, uint32_t iter) {

@@ -158,7 +158,7 @@ __global__ void __launch_bounds__(32 * WPC, WPC == 1 ? sweep_pipe_minb<MD>() : 2
         const int ps = c;                   // launch condition: one parameter set per chain, in chain order
         const int i0 = ly.i0[b], i1 = ly.i1[b];
         const bool last = ly.last[b] != 0;
-        const double rho = ly.rho[b], crho = sqrt(1.0 - rho * rho);
+        const double rho = layout_rho(ly, b, c, M), crho = sqrt(1.0 - rho * rho); // per task: a persistent warp changes block
         const GTile<NG> gt = g_tile_of<NG>(cx, ly, k, i1, last, 0, ps);
         double th[NPAR];
         {

@@ -48,7 +48,7 @@ __global__ void __launch_bounds__(32) sweep_sp_kernel(const DevCtx cx, const Lay
     const int ps = cx.pset[c];
     const int i0 = ly.i0[b], i1 = ly.i1[b];
     const bool last = ly.last[b] != 0;
-    const double rho = ly.rho[b], crho = sqrt(1.0 - rho * rho);
+    const double rho = layout_rho(ly, b, c, M), crho = sqrt(1.0 - rho * rho); // the four lanes of a chain share it
     const size_t gstr = P * 4;
 
     // ---- prefetch cursor (the tile after the one being computed) and its register buffer

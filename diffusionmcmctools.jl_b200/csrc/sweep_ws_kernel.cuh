@@ -360,7 +360,7 @@ __global__ void __launch_bounds__(SH::THREADS, 1) sweep_ws_kernel(const DevCtx c
         double acc = 0.0; // this lane's share of ll (A) / ll° (L)
         if (is_A) {
             // ---------------------------------------------------------------- A: K5, the accepted path's likelihood, the pCN refresh
-            const double rho = ly.rho[b], crho = sqrt(1.0 - rho * rho);
+            const double rho = layout_rho(ly, b, c, M), crho = sqrt(1.0 - rho * rho);
             // X two tiles ahead in registers: the tile's value at this lane's step
             WsCursor xc = cur_init();
             int jx = 0;

@@ -99,6 +99,25 @@ find_W_for_X = _fan(H.find_W_for_X)
 blocking_sweep = _fan(H.blocking_sweep)
 enable_guiding_cache = _fan(H.enable_guiding_cache)
 accpt_rate = _fan(H.accpt_rate)             # one vector (per block) per bucket: layouts differ between buckets
+enable_rho_adaptation, adapt_rho, disable_rho_adaptation = (_fan(f) for f in (H.enable_rho_adaptation, H.adapt_rho, H.disable_rho_adaptation))
+
+
+def rho_chains(hbe):
+    """per recording (global order): ρ [n_blocks] of each of its blocks (bb.ρ, src/biblock.jl:46; block counts differ between buckets)"""
+    per_bucket = [be.rho_chains for be in hbe.parts]
+    return [per_bucket[b][:, i].copy() for b, i in (hbe.he.where[r] for r in range(hbe.he.M_total))]
+
+
+def set_rho_chains(hbe, rho):
+    """rho: one value for every block of every recording, or one entry per recording in global order, each a value or [n_blocks]"""
+    if np.ndim(rho) == 0:
+        for be in hbe.parts:
+            H.set_rho_chains(be, rho)
+        return
+    if len(rho) != hbe.he.M_total:
+        raise ValueError("need one ρ entry per recording (%d), got %d" % (hbe.he.M_total, len(rho)))
+    for be, m in zip(hbe.parts, hbe.he.members):
+        H.set_rho_chains(be, np.stack([np.broadcast_to(np.asarray(rho[r], dtype=np.float64), (be.n_blocks,)) for r in m], axis=1))
 
 
 def fetch_ll(hbe):

@@ -164,8 +164,20 @@ class BiBlockView:
 
     def __init__(self, be, rec, blk):
         self.b, self.b_o = _BlockSide(be, rec, blk, 0), _BlockSide(be, rec, blk, 1)
-        self.rho = float(be.rho[blk])
         self._be, self._rec, self._blk = be, rec, blk
+
+    @property
+    def rho(self):
+        """bb.ρ (src/biblock.jl:46): the pCN memory of this block of this recording, read from the device"""
+        return float(self._be.ctx.get_rho_chains(self._be.layout)[self._blk, self._rec])
+
+    @rho.setter
+    def rho(self, value):
+        """sets this (recording, block) entry only; on a layout that adapts ρ the adaptation restarts from the new values"""
+        ctx, lay = self._be.ctx, self._be.layout
+        r = ctx.get_rho_chains(lay)
+        r[self._blk, self._rec] = float(value)
+        ctx.set_rho_chains(lay, r)
 
     @property
     def accpt_history(self):
@@ -268,6 +280,12 @@ class BlockEnsemble:
         self.ll_hist_len = ll_hist_len
         self.layout = se._alloc_layout()
         self.ctx.set_blocks(self.layout, self.ranges, self.rho, ll_hist_len=ll_hist_len)
+        self.rho_adaptation = None    # the settings of enable_rho_adaptation while ρ adapts
+
+    @property
+    def rho_chains(self):
+        """ρ of every block of every local recording, [n_blocks, M] (bb.ρ of each BiBlock, src/biblock.jl:46)"""
+        return self.ctx.get_rho_chains(self.layout)
 
     @property
     def recordings(self):
@@ -405,6 +423,33 @@ def enable_guiding_cache(be, enable=True):
     """Not in the reference: keep the v-independent part of the guiding term between sweeps (include/dmt.h, DESIGN.md §4).
     Use it for smoothing with blocking, where only the blocks' frozen end points change between recompute_guiding_term! calls."""
     be.ctx.enable_guiding_cache(be.layout, enable)
+
+
+def set_rho_chains(be, rho):
+    """bb.ρ of every BiBlock at once (src/biblock.jl:46): `rho` broadcasts to [n_blocks, M_total] over ALL recordings; each rank keeps
+    its own slice.  On a layout that adapts ρ the adaptation restarts from the new values."""
+    full = np.broadcast_to(np.asarray(rho, dtype=np.float64), (be.n_blocks, be.se.M_total))
+    be.ctx.set_rho_chains(be.layout, full[:, be.se.chain_lo:be.se.chain_hi])
+
+
+def enable_rho_adaptation(be, target=0.234, gamma0=1.0, decay=0.66, window=10, rho_min=0.0, rho_max=0.999):
+    """Not in the reference (the tutorials set ρ by hand and watch accpt_rate): adapt every (recording, block)'s ρ toward `target`
+    acceptance from its own decisions, on the device.  Call adapt_rho(be) after each accept_reject_proposal_path! during burn-in, then
+    disable_rho_adaptation(be): draws taken while ρ adapts are not from a fixed Markov kernel.  The rule is in include/dmt.h."""
+    be.ctx.set_rho_adaptation(be.layout, target, gamma0, decay, window, rho_min, rho_max)
+    be.rho_adaptation = dict(target=float(target), gamma0=float(gamma0), decay=float(decay), window=int(window),
+                             rho_min=float(rho_min), rho_max=float(rho_max))
+
+
+def adapt_rho(be):
+    """one adaptation step from the layout's last accept decisions (one kernel launch, no copy)"""
+    be.ctx.adapt_rho(be.layout)
+
+
+def disable_rho_adaptation(be):
+    """freeze ρ at its current values"""
+    be.ctx.set_rho_adaptation(be.layout, 0.0)
+    be.rho_adaptation = None
 
 
 def blocking_sweep(be, mcmciter):
@@ -572,16 +617,25 @@ class HistoryStreamer:
 
 
 # ---- checkpoint / resume (not in the reference, which keeps its state in Julia objects; SURVEY §5 / §8f item 3) -------------
+_ADAPT_KEYS = ("target", "gamma0", "decay", "window", "rho_min", "rho_max")
+
+
 def save_state(se, path, layouts=()):
     """Everything needed to continue a run bit-exactly: accepted and proposal X and W (resolved through the parity bits), the
-    accepted and proposal parameters θ / θ°, per layout the ll fields and the ll / accept histories, and the path moments
-    (PathMoments) when any were accumulated.  The counter-based generator needs no state beyond (seed, layout, iteration)."""
+    accepted and proposal parameters θ / θ°, per layout the ll fields, the ll / accept histories, ρ of every (block, recording) and,
+    while ρ adapts, the adaptation's settings and state, and the path moments (PathMoments) when any were accumulated.  The
+    counter-based generator needs no state beyond (seed, layout, iteration)."""
     ctx = se.ctx
     d = dict(X0=ctx.get_X(0), X1=ctx.get_X(1), W0=ctx.get_W(0), W1=ctx.get_W(1), theta=se.theta, theta_o=se.theta_o,
              n_pts=ctx.n_pts, tt=ctx.tt, chain_lo=se.chain_lo, chain_hi=se.chain_hi)
     for be in layouts:
         d["ll0_%d" % be.layout] = ctx.get_ll(be.layout, 0)
         d["ll1_%d" % be.layout] = ctx.get_ll(be.layout, 1)
+        d["rho_%d" % be.layout] = ctx.get_rho_chains(be.layout)
+        if be.rho_adaptation is not None:
+            a = be.rho_adaptation
+            d["rho_adapt_%d" % be.layout] = np.array([a[k] for k in _ADAPT_KEYS], dtype=np.float64)
+            d["rho_s_%d" % be.layout], d["rho_nacc_%d" % be.layout], d["rho_calls_%d" % be.layout] = ctx.get_rho_adaptation_state(be.layout)
         if be.ll_hist_len > 0:
             d["acc_hist_%d" % be.layout] = ctx.get_accept_history(be.layout, 0, be.ll_hist_len - 1)
             for s in (0, 1):
@@ -616,6 +670,14 @@ def load_state(se, path, layouts=()):
     for be in layouts:
         ctx.set_ll(be.layout, z["ll0_%d" % be.layout], 0)
         ctx.set_ll(be.layout, z["ll1_%d" % be.layout], 1)
+        if ("rho_%d" % be.layout) in z:
+            ctx.set_rho_chains(be.layout, z["rho_%d" % be.layout])
+            if ("rho_adapt_%d" % be.layout) in z:
+                a = z["rho_adapt_%d" % be.layout]
+                enable_rho_adaptation(be, **{k: (int(v) if k == "window" else float(v)) for k, v in zip(_ADAPT_KEYS, a)})
+                ctx.set_rho_adaptation_state(be.layout, z["rho_s_%d" % be.layout], z["rho_nacc_%d" % be.layout], int(z["rho_calls_%d" % be.layout]))
+            elif be.rho_adaptation is not None:
+                disable_rho_adaptation(be)
         if be.ll_hist_len > 0 and ("acc_hist_%d" % be.layout) in z:
             acc = z["acc_hist_%d" % be.layout]
             for i in range(be.ll_hist_len):

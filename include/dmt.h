@@ -103,11 +103,35 @@ int32_t dmt_set_obs(dmt_ctx *ctx, int32_t side, int32_t k0, int32_t k1, const do
 int32_t dmt_equalize_laws(dmt_ctx *ctx, int32_t store_mask, int32_t k0, int32_t k1, int32_t *changed);
 
 /* ---- block layouts (src/block_collection.jl:20-30; src/biblock.jl:49-62) ------------------------------------ */
-/* last[] NULL => only block n_blocks-1 is terminal (BlockCollection rule i==N).  rho[] per block (src/biblock.jl:46).
- * ll_hist_len: length of this layout's ll_history / accpt_history (src/biblock.jl:49-55); < 0 => dmt_config.ll_hist_len. */
+/* last[] NULL => only block n_blocks-1 is terminal (BlockCollection rule i==N).  rho[n_blocks] in [-1, 1]: the pCN memory of
+ * block b for every chain (each BiBlock owns its ρ, src/biblock.jl:46; the layout stores one per (block, chain)).
+ * ll_hist_len: length of this layout's ll_history / accpt_history (src/biblock.jl:49-55); < 0 => dmt_config.ll_hist_len.
+ * Re-registering a layout turns its ρ adaptation off. */
 int32_t dmt_set_blocks(dmt_ctx *ctx, int32_t layout, int32_t n_blocks, const int32_t *i0, const int32_t *i1, const double *rho,
                        const uint8_t *last, int32_t ll_hist_len);
+/* rho[n_blocks] for every chain: ρρ of BlockEnsemble (src/block_collection.jl:27) */
 int32_t dmt_set_rho(dmt_ctx *ctx, int32_t layout, const double *rho);
+/* bb.ρ of every BiBlock, one per (block, local chain): rho[n_blocks][M], every entry in [-1, 1] (src/biblock.jl:46).  On a layout
+ * that adapts ρ, dmt_set_rho and dmt_set_rho_chains restart the adaptation state from the new values (s from ρ, nacc = 0). */
+int32_t dmt_set_rho_chains(dmt_ctx *ctx, int32_t layout, const double *rho);
+int32_t dmt_get_rho_chains(dmt_ctx *ctx, int32_t layout, double *out /* [n_blocks][M] */);
+/* Adaptation of ρ toward a target acceptance rate: the tutorials tune bb.ρ by hand and watch accpt_rate (src/biblock.jl:46,232).
+ * Per (block, chain), from that chain's own decisions only, so a sharded run adapts exactly like the unsharded one.
+ * target <= 0: freeze ρ at its current values (adaptation off).  Otherwise 0 < target < 1, gamma0 > 0, 0.5 < decay <= 1, window >= 1,
+ * 0 <= rho_min < rho_max <= 1 (else DMT_ERR_ARG), and for every (b, c): u = clamp((ρ - rho_min) / (rho_max - rho_min), 1e-6, 1 - 1e-6),
+ * s = log(u / (1 - u)), nacc = 0; the layout's call counter restarts at 0. */
+int32_t dmt_set_rho_adaptation(dmt_ctx *ctx, int32_t layout, double target, double gamma0, double decay, int32_t window, double rho_min,
+                               double rho_max);
+/* One adaptation step after accept_reject_proposal_path!(be, i) (src/biblock.jl:121-127), ONE kernel launch: calls += 1;
+ * nacc += the layout's last accept decisions; when calls % window == 0, with n = calls / window and gamma = gamma0 n^-decay:
+ * s += gamma (target - nacc / window), ρ = rho_min + (rho_max - rho_min) / (1 + exp(-s)), nacc = 0.  Low acceptance raises ρ
+ * (smaller moves).  DMT_ERR_ARG when the layout does not adapt.  Draws made while ρ adapts are not from a fixed Markov kernel:
+ * keep samples from after the adaptation is frozen. */
+int32_t dmt_adapt_rho(dmt_ctx *ctx, int32_t layout);
+/* checkpoint / resume of the adaptation of bb.ρ (src/biblock.jl:46): s[n_blocks][M], nacc[n_blocks][M] (0 <= nacc < window), calls.  DMT_ERR_STATE when the
+ * layout does not adapt (set ρ with dmt_set_rho_chains and enable the adaptation first, then restore the state) */
+int32_t dmt_get_rho_adaptation_state(dmt_ctx *ctx, int32_t layout, double *s, int32_t *nacc, uint64_t *calls);
+int32_t dmt_set_rho_adaptation_state(dmt_ctx *ctx, int32_t layout, const double *s, const int32_t *nacc, uint64_t calls);
 
 /* ---- paths ---------------------------------------------------------------------------------------------------- */
 int32_t dmt_set_start(dmt_ctx *ctx, const double *x0 /* [d][M] */); /* XX[1].x[1] of u and u° */

@@ -496,8 +496,42 @@ accpt_rate(bc::DeviceBlockCollection, range) = [accpt_rate(bb, range) for bb in 
 ll_of_accepted(bb::DeviceBiBlock, i::Integer) = ll_of_accepted(bb.be, i)[bb.rec, bb.blk]                          # src/biblock.jl:222-225
 ll_of_accepted(bc::DeviceBlockCollection, i::Integer) = ll_of_accepted(bc.be, i)[bc.rec, :]                       # src/block_collection.jl:172
 
+# ---- the pCN memory: one ρ per (recording, block) as in the reference (bb.ρ, src/biblock.jl:46), and its adaptation toward a
+# target acceptance rate on the device (include/dmt.h).  Burn-in: blocking_sweep!; accept_reject_proposal_path!; adapt_rho!; then
+# disable_rho_adaptation! before keeping samples (draws taken while ρ adapts are not from a fixed Markov kernel).
+"""    rho_chains(be) -> Matrix (M, n_blocks): ρ of every block of every recording"""
+function rho_chains(be::DBE)
+    ρ = Matrix{Float64}(undef, be.se.M, be.n_blocks)
+    check(be.se.ctx, ccall((:dmt_get_rho_chains, libdmt), Int32, (Ptr{Cvoid}, Int32, Ptr{Float64}), be.se.ctx, be.layout, ρ))
+    ρ
+end
+"""    set_rho_chains!(be, ρ): ρ broadcasts to (M, n_blocks); on an adapting layout the adaptation restarts from the new values"""
+function set_rho_chains!(be::DBE, ρ)
+    r = Matrix{Float64}(undef, be.se.M, be.n_blocks)
+    r .= ρ
+    check(be.se.ctx, ccall((:dmt_set_rho_chains, libdmt), Int32, (Ptr{Cvoid}, Int32, Ptr{Float64}), be.se.ctx, be.layout, r))
+end
+enable_rho_adaptation!(be::DBE; target=0.234, γ0=1.0, decay=0.66, window=10, ρmin=0.0, ρmax=0.999) =
+    check(be.se.ctx, ccall((:dmt_set_rho_adaptation, libdmt), Int32, (Ptr{Cvoid}, Int32, Float64, Float64, Float64, Int32, Float64, Float64),
+                           be.se.ctx, be.layout, target, γ0, decay, window, ρmin, ρmax))
+disable_rho_adaptation!(be::DBE) =
+    check(be.se.ctx, ccall((:dmt_set_rho_adaptation, libdmt), Int32, (Ptr{Cvoid}, Int32, Float64, Float64, Float64, Int32, Float64, Float64),
+                           be.se.ctx, be.layout, 0.0, 0.0, 0.0, 0, 0.0, 0.0))
+adapt_rho!(be::DBE) = check(be.se.ctx, ccall((:dmt_adapt_rho, libdmt), Int32, (Ptr{Cvoid}, Int32), be.se.ctx, be.layout))
+# bb.ρ reads and writes that one (recording, block) entry
+Base.getproperty(bb::DeviceBiBlock, s::Symbol) =
+    s === :ρ ? rho_chains(getfield(bb, :be))[getfield(bb, :rec), getfield(bb, :blk)] : getfield(bb, s)
+function Base.setproperty!(bb::DeviceBiBlock, s::Symbol, v)
+    s === :ρ || return setfield!(bb, s, v)
+    be = getfield(bb, :be)
+    r = rho_chains(be)
+    r[getfield(bb, :rec), getfield(bb, :blk)] = v
+    set_rho_chains!(be, r)
+end
+
 export DeviceEnsemble, DeviceBlockEnsemble, DeviceBlockCollection, DeviceBiBlock, upload_aux!, get_paths, get_X, get_W, trajectories,
     wiener_trajectories, pack_paths, pack_noise, recordings, blocks, blocking_sweep!, enable_guiding_cache!, path_moments_add!,
-    path_moments_reset!, path_moments, set_path_moments!, pset_path_moments
+    path_moments_reset!, path_moments, set_path_moments!, pset_path_moments, rho_chains, set_rho_chains!, enable_rho_adaptation!,
+    disable_rho_adaptation!, adapt_rho!
 
 end # module
