@@ -64,20 +64,26 @@ bool model_dims(int model, ModelDims &md) {
     return false;
 }
 
+// Ordering rule: every copy and fill goes on the context's stream (ctx->stream), in order with the kernels that use the memory.
+// Only the asynchronous read-backs (dmt_snapshot_paths_async, dmt_histories_async) run on copy_stream, behind an event.  The
+// context's stream is non-blocking: nothing may go on the legacy default stream, which it does not order against.  An entry point
+// that hands host memory to an async copy waits for ctx->stream before it returns.
 template <class T> struct DevBuf {
     T *p = nullptr;
     size_t n = 0;
-    void alloc(size_t count, bool zero = true) {
+    void alloc_uninit(size_t count) {
         release();
         n = count;
-        if (count) {
-            CK(cudaMalloc(&p, count * sizeof(T)));
-            if (zero) { // the memset runs on the legacy stream, which the contexts' non-blocking streams do NOT order against:
-                        // wait for it here, or the first kernels on ctx->stream may see (or be overwritten by) the zero fill
-                CK(cudaMemsetAsync(p, 0, count * sizeof(T), cudaStreamLegacy));
-                CK(cudaStreamSynchronize(cudaStreamLegacy));
-            }
-        }
+        if (count) CK(cudaMalloc(&p, count * sizeof(T)));
+    }
+    void alloc(size_t count, cudaStream_t stream) { // zero-filled
+        alloc_uninit(count);
+        if (count) CK(cudaMemsetAsync(p, 0, count * sizeof(T), stream));
+    }
+    // the contents of `host`; the storage is kept when the size matches
+    void upload(const std::vector<T> &host, cudaStream_t stream) {
+        if (n != host.size()) alloc_uninit(host.size());
+        if (n) CK(cudaMemcpyAsync(p, host.data(), n * sizeof(T), cudaMemcpyHostToDevice, stream));
     }
     void release() {
         if (p) cudaFree(p);
@@ -159,7 +165,7 @@ struct dmt_ctx {
     ModelDims md{};
     int D = 0, DW = 0, NPAR = 0, NH = 0, NG = 0, NAUX = 0, NOBS = 0;
     int K = 0, M = 0, P = 0, m = 0, NT = 0, NTb = 0, S = 0, NP = 0;
-    std::vector<int> nsteps, tile0, step0, pt0, ppb_tile0;
+    std::vector<int> nsteps, tile0, step0, pt0, ppb_tile0, pset; // host copies of the d_ maps below
     cudaStream_t stream = nullptr;
     DevCtx dev{};
     std::vector<Layout> layouts;
@@ -208,7 +214,7 @@ struct dmt_ctx {
     DevBuf<int> d_pm_cs, d_pm_chains;
 
     double *scratch(size_t n) {
-        if (d_scratch.n < n) d_scratch.alloc(n, false);
+        if (d_scratch.n < n) d_scratch.alloc_uninit(n);
         return d_scratch.p;
     }
 };
@@ -319,8 +325,8 @@ template <class MD, bool LAZY> void launch_sweep_pipe(dmt_ctx *c, Layout &L, con
         ++g_launches, sweep_pipe_kernel<MD, LAZY, 1><<<dim3((unsigned)groups, L.nb, 1), 32, smem, c->stream>>>(c->dev, L.dev, fa, PipeSched{});
         return;
     }
-    if (L.d_ticket.n != 1 + units) L.d_ticket.alloc(1 + units, false);
-    if (L.d_hand.n != (size_t)(MD::D + 3) * units * 32) L.d_hand.alloc((size_t)(MD::D + 3) * units * 32, false);
+    if (L.d_ticket.n != 1 + units) L.d_ticket.alloc_uninit(1 + units);
+    if (L.d_hand.n != (size_t)(MD::D + 3) * units * 32) L.d_hand.alloc_uninit((size_t)(MD::D + 3) * units * 32);
     CK(cudaMemsetAsync(L.d_ticket.p, 0, sizeof(unsigned) * (1 + units), c->stream));
     const PipeSched sc{L.d_task.p, (int)(L.d_task.n * groups), L.d_ticket.p, L.d_hand.p};
     ++g_launches, sweep_pipe_kernel<MD, LAZY, WPC><<<(unsigned)(n / WPC), 32 * WPC, WPC * smem, c->stream>>>(c->dev, L.dev, fa, sc);
@@ -422,7 +428,7 @@ template <class MD> void launch_bwd_model(dmt_ctx *c, Layout &L, const BwdArgs &
     const int nz = c->cfg.two_sided_laws ? 2 : 1;
     if (c->bwd_solver == 1) { // upstream's solver (tsit5_kernel.cuh); the guiding cache's probes need the fixed-grid discretisation
         REQUIRE(!ba.use_override, DMT_ERR_UNSUPPORTED, "the guiding cache needs the RK4 backward filter (its F is affine in v only there)");
-        if (c->d_steps.n < 2) c->d_steps.alloc(2);
+        if (c->d_steps.n < 2) c->d_steps.alloc(2, c->stream);
         CK(cudaMemsetAsync(c->d_steps.p, 0, 2 * sizeof(int), c->stream));
         Tsit5Args ta{ba.side_mask, c->bwd_reltol, c->bwd_abstol, c->d_steps.p};
         ++g_launches, bwd_tsit5_kernel<MD><<<pset_grid(c, L.nb, 32, nz), 32, 0, c->stream>>>(c->dev, L.dev, ta);
@@ -502,26 +508,22 @@ void cache_build(dmt_ctx *c, Layout &L) {
     const size_t P = c->P, NF = c->D + c->D * c->D, NC = 1 + c->D + c->NH;
     const size_t nt[2] = {(size_t)c->NT, (size_t)std::max(c->NTb, 1)};
     for (int st = 0; st < 2; st++) {
-        if (L.d_Gl[st].n != nt[st] * c->NG * P * 4) L.d_Gl[st].alloc(nt[st] * c->NG * P * 4);
-        if (L.d_FP[st].n != fp_tiles_padded(nt[st]) * NF * P * 4) L.d_FP[st].alloc(fp_tiles_padded(nt[st]) * NF * P * 4);
-        if (L.d_c0l[st].n != (size_t)c->K * P) L.d_c0l[st].alloc((size_t)c->K * P);
+        if (L.d_Gl[st].n != nt[st] * c->NG * P * 4) L.d_Gl[st].alloc(nt[st] * c->NG * P * 4, c->stream);
+        if (L.d_FP[st].n != fp_tiles_padded(nt[st]) * NF * P * 4) L.d_FP[st].alloc(fp_tiles_padded(nt[st]) * NF * P * 4, c->stream);
+        if (L.d_c0l[st].n != (size_t)c->K * P) L.d_c0l[st].alloc((size_t)c->K * P, c->stream);
         L.dev.FP[st] = L.d_FP[st].p;
     }
-    if (L.d_cq.n != (size_t)L.nb * NC * P) L.d_cq.alloc((size_t)L.nb * NC * P);
+    if (L.d_cq.n != (size_t)L.nb * NC * P) L.d_cq.alloc((size_t)L.nb * NC * P, c->stream);
     L.dev.cq = L.d_cq.p;
-    if (L.d_vlast.n != (size_t)L.nb * c->D * P) L.d_vlast.alloc((size_t)L.nb * c->D * P, false);
+    // "no end point seen yet": NaN compares unequal to everything, so the first apply after a (re)build materialises every block
+    L.d_vlast.upload(std::vector<double>((size_t)L.nb * c->D * P, NAN), c->stream);
+    CK(cudaStreamSynchronize(c->stream));
     L.dev.v_last = L.d_vlast.p;
-    {   // "no end point seen yet": NaN compares unequal to everything, so the first apply after a (re)build materialises every block
-        std::vector<double> nan_fill(L.d_vlast.n, NAN);
-        CK(cudaMemcpyAsync(L.d_vlast.p, nan_fill.data(), sizeof(double) * nan_fill.size(), cudaMemcpyHostToDevice, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-    }
     {
         std::vector<int> bk(c->K, 0);
         for (int b = 0; b < L.nb; b++)
             for (int k = L.i0[b]; k <= L.i1[b]; k++) bk[k] = b;
-        if (L.d_blk_of_k.n != (size_t)c->K) L.d_blk_of_k.alloc(c->K);
-        CK(cudaMemcpyAsync(L.d_blk_of_k.p, bk.data(), sizeof(int) * c->K, cudaMemcpyHostToDevice, c->stream));
+        L.d_blk_of_k.upload(bk, c->stream);
         CK(cudaStreamSynchronize(c->stream));
         L.dev.blk_of_k = L.d_blk_of_k.p;
     }
@@ -530,7 +532,7 @@ void cache_build(dmt_ctx *c, Layout &L) {
     const int D = c->D, nruns = 1 + 2 * D + D * (D - 1) / 2;
     const double s = 8.0; // probe scale (a power of two: exact scaling)
     DevBuf<double> Crun;
-    Crun.alloc((size_t)nruns * L.nb * P);
+    Crun.alloc((size_t)nruns * L.nb * P, c->stream);
     const dim3 g0((c->P + 127) / 128, c->NT), g1((c->P + 127) / 128, std::max(c->NTb, 1));
     std::vector<std::vector<double>> probes;
     probes.push_back(std::vector<double>(6, 0.0));
@@ -636,9 +638,9 @@ void rebuild_ppb_store(dmt_ctx *c) {
     c->ppb_tile0 = t0;
     c->NTb = nt;
     CK(cudaStreamSynchronize(c->stream)); // kernels in flight still read the old map / the old store
-    CK(cudaMemcpy(c->d_ppb_tile0.p, t0.data(), sizeof(int) * c->K, cudaMemcpyHostToDevice));
+    c->d_ppb_tile0.upload(t0, c->stream);
     for (int s = 0; s < (c->cfg.two_sided_laws ? 2 : 1); s++) {
-        c->d_G[s][1].alloc((size_t)std::max(nt, 1) * c->NG * c->P * 4);
+        c->d_G[s][1].alloc((size_t)std::max(nt, 1) * c->NG * c->P * 4, c->stream);
         c->dev.G[s][1] = c->d_G[s][1].p;
     }
     c->dev.NTb = nt;
@@ -647,17 +649,15 @@ void rebuild_ppb_store(dmt_ctx *c) {
         for (int k = 0; k < c->K; k++)
             if (t0[k] >= 0)
                 for (int q = 0; q < (c->nsteps[k] + 3) / 4; q++) kt[t0[k] + q] = k;
-        c->d_k_of_ppbtile.alloc(kt.size());
-        CK(cudaMemcpy(c->d_k_of_ppbtile.p, kt.data(), sizeof(int) * kt.size(), cudaMemcpyHostToDevice));
-        CK(cudaStreamSynchronize(cudaStreamLegacy)); // pageable H2D copies return before the DMA lands; ctx->stream does not order against them
+        c->d_k_of_ppbtile.upload(kt, c->stream);
         invalidate_caches(c);
     }
 }
 
 void fill_stats(dmt_ctx *c, Layout &L, double *host_out /* [2+3nb] */) {
     const int ncta = (c->M + 255) / 256;
-    if (c->d_partial.n < (size_t)3 * L.nb * ncta) c->d_partial.alloc((size_t)3 * L.nb * ncta);
-    if (c->d_stats.n < (size_t)(2 + 3 * L.nb)) c->d_stats.alloc(2 + 3 * L.nb);
+    if (c->d_partial.n < (size_t)3 * L.nb * ncta) c->d_partial.alloc((size_t)3 * L.nb * ncta, c->stream);
+    if (c->d_stats.n < (size_t)(2 + 3 * L.nb)) c->d_stats.alloc(2 + 3 * L.nb, c->stream);
     ++g_launches, reduce_stats_kernel<<<dim3(ncta, L.nb), 256, 0, c->stream>>>(L.d_ll.p, L.d_last_acc.p, c->M, L.nb, c->d_partial.p);
     CK(cudaGetLastError());
     ++g_launches, finish_stats_kernel<<<1, 64, 0, c->stream>>>(c->d_partial.p, ncta, L.nb, c->d_stats.p);
@@ -791,46 +791,38 @@ int32_t dmt_create(const dmt_config *cfg, const int32_t *n_pts, const double *tt
                 sq[(size_t)c->tile0[k] * 4 + j] = std::sqrt(h);
             }
         c->ppb_tile0.assign(K, -1);
-        std::vector<int> pset(c->M);
+        c->pset.resize(c->M);
         for (int i = 0; i < c->M; i++) {
-            pset[i] = pset_of_chain ? pset_of_chain[i] : (c->P == c->M ? i : 0);
-            REQUIRE(pset[i] >= 0 && pset[i] < c->P, DMT_ERR_ARG, "pset_of_chain entry out of range");
+            c->pset[i] = pset_of_chain ? pset_of_chain[i] : (c->P == c->M ? i : 0);
+            REQUIRE(c->pset[i] >= 0 && c->pset[i] < c->P, DMT_ERR_ARG, "pset_of_chain entry out of range");
             REQUIRE(pset_of_chain || c->P == c->M || c->P == 1, DMT_ERR_ARG, "pset_of_chain required when 1 < P < M");
         }
         {
             bool ident = (c->P == c->M);
-            for (int i = 0; i < c->M && ident; i++) ident = (pset[i] == i);
+            for (int i = 0; i < c->M && ident; i++) ident = (c->pset[i] == i);
             c->pipe_ok = ident;
         }
-        c->d_tile0.alloc(K + 1); c->d_step0.alloc(K + 1); c->d_pt0.alloc(K + 1); c->d_nsteps.alloc(K); c->d_ppb_tile0.alloc(K);
-        c->d_pset.alloc(c->M); c->d_dt.alloc(dt.size()); c->d_sqdt.alloc(sq.size());
-        CK(cudaMemcpy(c->d_tile0.p, c->tile0.data(), sizeof(int) * (K + 1), cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(c->d_step0.p, c->step0.data(), sizeof(int) * (K + 1), cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(c->d_pt0.p, c->pt0.data(), sizeof(int) * (K + 1), cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(c->d_nsteps.p, c->nsteps.data(), sizeof(int) * K, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(c->d_ppb_tile0.p, c->ppb_tile0.data(), sizeof(int) * K, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(c->d_pset.p, pset.data(), sizeof(int) * c->M, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(c->d_dt.p, dt.data(), sizeof(double) * dt.size(), cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(c->d_sqdt.p, sq.data(), sizeof(double) * sq.size(), cudaMemcpyHostToDevice));
-        CK(cudaStreamSynchronize(cudaStreamLegacy)); // pageable H2D copies return before the DMA lands; ctx->stream does not order against them
+        c->d_tile0.upload(c->tile0, c->stream); c->d_step0.upload(c->step0, c->stream); c->d_pt0.upload(c->pt0, c->stream);
+        c->d_nsteps.upload(c->nsteps, c->stream); c->d_ppb_tile0.upload(c->ppb_tile0, c->stream); c->d_pset.upload(c->pset, c->stream);
+        c->d_dt.upload(dt, c->stream); c->d_sqdt.upload(sq, c->stream);
 
         // ---- SoA containers (SamplingPair: accepted + proposal buffers)
         const size_t M = c->M, P = c->P, NT = c->NT;
         const size_t xb = NT * c->D * M * 4, wb = NT * c->DW * M * 4, x0b = (size_t)K * c->D * M;
-        c->d_X.alloc(2 * xb); c->d_W.alloc(2 * wb); c->d_X0.alloc(2 * x0b);
-        c->d_parX.alloc((size_t)K * M); c->d_parW.alloc((size_t)K * M);
+        c->d_X.alloc(2 * xb, c->stream); c->d_W.alloc(2 * wb, c->stream); c->d_X0.alloc(2 * x0b, c->stream);
+        c->d_parX.alloc((size_t)K * M, c->stream); c->d_parW.alloc((size_t)K * M, c->stream);
         const int nslot = cfg->two_sided_laws ? 2 : 1;
-        for (int st = 0; st < 2; st++) c->d_parP[st].alloc((size_t)K * P);
+        for (int st = 0; st < 2; st++) c->d_parP[st].alloc((size_t)K * P, c->stream);
         for (int s = 0; s < nslot; s++) {
-            c->d_G[s][0].alloc(NT * c->NG * P * 4);
-            c->d_G[s][1].alloc((size_t)c->NG * P * 4);
+            c->d_G[s][0].alloc(NT * c->NG * P * 4, c->stream);
+            c->d_G[s][1].alloc((size_t)c->NG * P * 4, c->stream);
             for (int st = 0; st < 2; st++) {
-                c->d_c0[s][st].alloc((size_t)K * P);
-                c->d_theta[s][st].alloc((size_t)K * c->NPAR * P);
-                c->d_aux[s][st].alloc((size_t)K * c->NAUX * P);
+                c->d_c0[s][st].alloc((size_t)K * P, c->stream);
+                c->d_theta[s][st].alloc((size_t)K * c->NPAR * P, c->stream);
+                c->d_aux[s][st].alloc((size_t)K * c->NAUX * P, c->stream);
             }
-            c->d_obs[s].alloc((size_t)K * c->NOBS * P);
-            c->d_vart[s].alloc((size_t)K * c->D * P);
+            c->d_obs[s].alloc((size_t)K * c->NOBS * P, c->stream);
+            c->d_vart[s].alloc((size_t)K * c->D * P, c->stream);
         }
         DevCtx &d = c->dev;
         d.M = c->M; d.P = c->P; d.K = K; d.NT = c->NT; d.NTb = 0; d.m = c->m; d.two_sided = cfg->two_sided_laws ? 1 : 0;
@@ -840,8 +832,7 @@ int32_t dmt_create(const dmt_config *cfg, const int32_t *n_pts, const double *tt
             std::vector<int> kt(c->NT, 0);
             for (int k = 0; k < K; k++)
                 for (int t = c->tile0[k]; t < c->tile0[k + 1]; t++) kt[t] = k;
-            c->d_k_of_tile.alloc(c->NT);
-            CK(cudaMemcpy(c->d_k_of_tile.p, kt.data(), sizeof(int) * c->NT, cudaMemcpyHostToDevice));
+            c->d_k_of_tile.upload(kt, c->stream);
             d.k_of_tile = c->d_k_of_tile.p;
         }
         d.X = c->d_X.p; d.W = c->d_W.p; d.X0 = c->d_X0.p; d.Xbuf = xb; d.Wbuf = wb; d.X0buf = x0b;
@@ -856,7 +847,7 @@ int32_t dmt_create(const dmt_config *cfg, const int32_t *n_pts, const double *tt
         }
         d.eps = cfg->artificial_noise; d.seed = cfg->seed; d.chain_offset = (uint32_t)cfg->chain_offset;
         c->layouts.resize(cfg->n_layouts);
-        CK(cudaDeviceSynchronize());
+        CK(cudaStreamSynchronize(c->stream));
         *out = c;
         return DMT_OK;
     } catch (const DmtError &e) {
@@ -881,6 +872,7 @@ int32_t dmt_destroy(dmt_ctx *ctx) {
     if (ctx->copy_stream) { cudaStreamSynchronize(ctx->copy_stream); cudaStreamDestroy(ctx->copy_stream); }
     if (ctx->ev_gathered) cudaEventDestroy(ctx->ev_gathered);
     if (ctx->ev_copied) cudaEventDestroy(ctx->ev_copied);
+    if (ctx->ev_hist) cudaEventDestroy(ctx->ev_hist);
     if (ctx->stream) { cudaStreamSynchronize(ctx->stream); cudaStreamDestroy(ctx->stream); }
     delete ctx;
     return DMT_OK;
@@ -937,7 +929,7 @@ int32_t dmt_set_aux_linearised(dmt_ctx *ctx, int32_t side, int32_t store, int32_
         if (side == 0) { ensure_W(ctx); invalidate_caches(ctx); } // the accepted laws change: cached guiding terms are stale
         REQUIRE(store == 0 || store == 1, DMT_ERR_ARG, "store must be 0 (PP) or 1 (PPb)");
         const size_t per_k = (size_t)ctx->D * ctx->P, n = (size_t)(k1 - k0 + 1) * per_k;
-        if (ctx->d_xbar[store].n < (size_t)ctx->K * per_k) { ctx->d_xbar[store].alloc((size_t)ctx->K * per_k); ctx->xbar_set[store].assign(ctx->K, 0); }
+        if (ctx->d_xbar[store].n < (size_t)ctx->K * per_k) { ctx->d_xbar[store].alloc((size_t)ctx->K * per_k, ctx->stream); ctx->xbar_set[store].assign(ctx->K, 0); }
         double *tmp = ctx->d_xbar[store].p + (size_t)k0 * per_k;
         if (xbar) { // new linearisation points: keep them on the device
             CK(cudaMemcpyAsync(tmp, xbar, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
@@ -975,7 +967,7 @@ int32_t dmt_equalize_laws(dmt_ctx *ctx, int32_t store_mask, int32_t k0, int32_t 
     return guarded(ctx, [&] {
         check_law_side(ctx, 1); check_range(ctx, k0, k1);
         dim3 grid = pset_grid(ctx, k1 - k0 + 1, 128);
-        if (ctx->d_flag.n < 1) ctx->d_flag.alloc(1);
+        if (ctx->d_flag.n < 1) ctx->d_flag.alloc(1, ctx->stream);
         CK(cudaMemsetAsync(ctx->d_flag.p, 0, sizeof(int), ctx->stream));
         for (int st = 0; st < 2; st++) {
             if (!((store_mask >> st) & 1)) continue;
@@ -1013,24 +1005,15 @@ int32_t dmt_set_blocks(dmt_ctx *ctx, int32_t layout, int32_t n_blocks, const int
         const size_t M = ctx->M;
         L.nb = n_blocks;
         L.i0.assign(i0, i0 + n_blocks); L.i1.assign(i1, i1 + n_blocks); L.last = lst;
-        L.d_i0.alloc(n_blocks); L.d_i1.alloc(n_blocks); L.d_last.alloc(n_blocks); L.d_rho.alloc(n_blocks * M);
-        L.d_ll.alloc(2 * n_blocks * M); L.d_ok.alloc(n_blocks * M); L.d_last_acc.alloc(n_blocks * M);
-        CK(cudaMemcpy(L.d_i0.p, i0, sizeof(int) * n_blocks, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(L.d_i1.p, i1, sizeof(int) * n_blocks, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(L.d_last.p, lst.data(), n_blocks, cudaMemcpyHostToDevice));
-        {
-            const std::vector<double> rr = rho_per_chain(ctx, n_blocks, rho);
-            CK(cudaMemcpy(L.d_rho.p, rr.data(), sizeof(double) * rr.size(), cudaMemcpyHostToDevice));
-        }
+        L.d_i0.upload(L.i0, ctx->stream); L.d_i1.upload(L.i1, ctx->stream); L.d_last.upload(L.last, ctx->stream);
+        L.d_rho.upload(rho_per_chain(ctx, n_blocks, rho), ctx->stream);
+        L.d_ll.upload(std::vector<double>(2 * n_blocks * M, -INFINITY), ctx->stream); // Block ctor: ll = -Inf (src/block.jl:74)
+        L.d_ok.alloc(n_blocks * M, ctx->stream); L.d_last_acc.alloc(n_blocks * M, ctx->stream);
         L.adapt = false;
         L.d_ad_s.release(); L.d_ad_nacc.release();
-        {   // Block ctor: ll = -Inf (src/block.jl:74)
-            std::vector<double> ninf(2 * n_blocks * M, -INFINITY);
-            CK(cudaMemcpy(L.d_ll.p, ninf.data(), sizeof(double) * ninf.size(), cudaMemcpyHostToDevice));
-        }
         const int hl_req = ll_hist_len >= 0 ? ll_hist_len : ctx->cfg.ll_hist_len;
         const size_t hl = hl_req > 0 ? hl_req : 0;
-        if (hl) { L.d_acc_hist.alloc(hl * n_blocks * M); L.d_ll_hist.alloc(hl * 2 * n_blocks * M); }
+        if (hl) { L.d_acc_hist.alloc(hl * n_blocks * M, ctx->stream); L.d_ll_hist.alloc(hl * 2 * n_blocks * M, ctx->stream); }
         L.dev.nb = n_blocks; L.dev.id = layout;
         L.dev.i0 = L.d_i0.p; L.dev.i1 = L.d_i1.p; L.dev.last = L.d_last.p; L.dev.rho = L.d_rho.p;
         L.dev.ll = L.d_ll.p; L.dev.ok = L.d_ok.p; L.dev.last_acc = L.d_last_acc.p;
@@ -1043,13 +1026,13 @@ int32_t dmt_set_blocks(dmt_ctx *ctx, int32_t layout, int32_t n_blocks, const int
                     if (i0[b] + j <= i1[b]) task.push_back(b + 64 * j);
                 if (task.size() == n0) break;
             }
-            L.d_task.alloc(task.size(), false);
-            CK(cudaMemcpy(L.d_task.p, task.data(), sizeof(int) * task.size(), cudaMemcpyHostToDevice));
+            L.d_task.upload(task, ctx->stream);
         }
         L.set = true;
         L.cache_enabled = false; L.cache_valid = false;
         cache_set_private(L, false);
         rebuild_ppb_store(ctx);
+        CK(cudaStreamSynchronize(ctx->stream));
     });
 }
 
@@ -1094,7 +1077,7 @@ int32_t dmt_set_rho_adaptation(dmt_ctx *ctx, int32_t layout, double target, doub
         L.ad_target = target; L.ad_gamma0 = gamma0; L.ad_decay = decay; L.ad_window = window;
         L.ad_rho_min = rho_min; L.ad_rho_max = rho_max;
         const size_t n = (size_t)L.nb * ctx->M;
-        if (L.d_ad_s.n != n) { L.d_ad_s.alloc(n, false); L.d_ad_nacc.alloc(n, false); }
+        if (L.d_ad_s.n != n) { L.d_ad_s.alloc_uninit(n); L.d_ad_nacc.alloc_uninit(n); }
         std::vector<double> rho(n);
         CK(cudaMemcpyAsync(rho.data(), L.d_rho.p, sizeof(double) * n, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
@@ -1167,7 +1150,7 @@ static void xfer_paths(dmt_ctx *ctx, int side, double *host, bool is_x, bool upl
     }
     const size_t n = is_x ? (size_t)ctx->NP * ctx->D * ctx->M : (size_t)ctx->S * ctx->DW * ctx->M;
     DevBuf<double> nat;
-    nat.alloc(n, false);
+    nat.alloc_uninit(n);
     if (upload) CK(cudaMemcpyAsync(nat.p, host, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     dim3 grid = chain_grid(ctx, ctx->K, 128);
     if (is_x) ++g_launches, xfer_X_kernel<<<grid, 128, 0, ctx->stream>>>(ctx->dev, side, ctx->D, nat.p, upload ? 1 : 0);
@@ -1181,22 +1164,27 @@ int32_t dmt_get_X(dmt_ctx *ctx, int32_t side, double *X) { return guarded(ctx, [
 int32_t dmt_set_W(dmt_ctx *ctx, int32_t side, const double *W) { return guarded(ctx, [&] { xfer_paths(ctx, side, (double *)W, false, true); }); }
 int32_t dmt_get_W(dmt_ctx *ctx, int32_t side, double *W) { return guarded(ctx, [&] { xfer_paths(ctx, side, W, false, false); }); }
 
+// the stream of the asynchronous read-backs and its events, created on first use
+static void ensure_copy_stream(dmt_ctx *ctx) {
+    if (ctx->copy_stream) return;
+    CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+    CK(cudaEventCreateWithFlags(&ctx->ev_gathered, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&ctx->ev_copied, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&ctx->ev_hist, cudaEventDisableTiming));
+    CK(cudaEventRecord(ctx->ev_copied, ctx->copy_stream));
+}
+
 int32_t dmt_snapshot_paths_async(dmt_ctx *ctx, int32_t side, int32_t n_sel, const int32_t *chains, double *host_out) {
     return guarded(ctx, [&] {
         check_side(ctx, side);
         REQUIRE(n_sel >= 1 && chains && host_out, DMT_ERR_ARG, "bad snapshot arguments");
         for (int i = 0; i < n_sel; i++) REQUIRE(chains[i] >= 0 && chains[i] < ctx->M, DMT_ERR_ARG, "chain index out of range");
-        if (!ctx->copy_stream) {
-            CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-            CK(cudaEventCreateWithFlags(&ctx->ev_gathered, cudaEventDisableTiming));
-            CK(cudaEventCreateWithFlags(&ctx->ev_copied, cudaEventDisableTiming));
-            CK(cudaEventRecord(ctx->ev_copied, ctx->copy_stream));
-        }
+        ensure_copy_stream(ctx);
         const size_t n = (size_t)ctx->NP * ctx->D * n_sel;
         // the staging buffer is reused: the gather may not start before the previous snapshot has left the device
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_copied, 0));
-        if (ctx->d_snap.n < n) { CK(cudaStreamSynchronize(ctx->copy_stream)); ctx->d_snap.alloc(n, false); }
-        if (ctx->d_snap_sel.n < (size_t)n_sel) { CK(cudaStreamSynchronize(ctx->copy_stream)); ctx->d_snap_sel.alloc(n_sel, false); }
+        if (ctx->d_snap.n < n) { CK(cudaStreamSynchronize(ctx->copy_stream)); ctx->d_snap.alloc_uninit(n); }
+        if (ctx->d_snap_sel.n < (size_t)n_sel) { CK(cudaStreamSynchronize(ctx->copy_stream)); ctx->d_snap_sel.alloc_uninit(n_sel); }
         CK(cudaMemcpyAsync(ctx->d_snap_sel.p, chains, sizeof(int) * n_sel, cudaMemcpyHostToDevice, ctx->stream));
         ++g_launches, gather_X_kernel<<<dim3((n_sel + 63) / 64, ctx->K), 64, 0, ctx->stream>>>(ctx->dev, side, ctx->D, ctx->d_snap_sel.p, n_sel, ctx->d_snap.p);
         CK(cudaGetLastError());
@@ -1216,8 +1204,8 @@ static void get_paths_of(dmt_ctx *ctx, int side, int n_sel, const int32_t *chain
     const size_t n = (is_x ? (size_t)ctx->NP * ctx->D : (size_t)ctx->S * ctx->DW) * n_sel;
     DevBuf<double> d;
     DevBuf<int> sel;
-    d.alloc(n, false);
-    sel.alloc(n_sel, false);
+    d.alloc_uninit(n);
+    sel.alloc_uninit(n_sel);
     CK(cudaMemcpyAsync(sel.p, chains, sizeof(int) * n_sel, cudaMemcpyHostToDevice, ctx->stream));
     const dim3 grid((n_sel + 63) / 64, ctx->K);
     if (is_x) ++g_launches, gather_X_kernel<<<grid, 64, 0, ctx->stream>>>(ctx->dev, side, ctx->D, sel.p, n_sel, d.p);
@@ -1238,13 +1226,7 @@ int32_t dmt_histories_async(dmt_ctx *ctx, int32_t layout, uint32_t it0, uint32_t
     return guarded(ctx, [&] {
         Layout &L = layout_of(ctx, layout);
         REQUIRE((host_ll || host_acc) && it0 <= it1 && it1 < (uint32_t)L.dev.hist_len, DMT_ERR_ARG, "bad history range");
-        if (!ctx->copy_stream) {
-            CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-            CK(cudaEventCreateWithFlags(&ctx->ev_gathered, cudaEventDisableTiming));
-            CK(cudaEventCreateWithFlags(&ctx->ev_copied, cudaEventDisableTiming));
-            CK(cudaEventRecord(ctx->ev_copied, ctx->copy_stream));
-        }
-        if (!ctx->ev_hist) CK(cudaEventCreateWithFlags(&ctx->ev_hist, cudaEventDisableTiming));
+        ensure_copy_stream(ctx);
         const size_t per = (size_t)L.nb * ctx->M, n = (size_t)(it1 - it0 + 1);
         CK(cudaEventRecord(ctx->ev_hist, ctx->stream));
         CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_hist, 0));
@@ -1419,7 +1401,7 @@ static void swap_impl(dmt_ctx *ctx, int32_t layout, int32_t what, const uint8_t 
     if (mask) {
         REQUIRE(!(what & DMT_SWAP_PP) || ctx->P == ctx->M, DMT_ERR_UNSUPPORTED, "masked swap_PP! needs n_psets == n_chains");
         const size_t n = (size_t)ctx->M * (per_block ? L.nb : 1);
-        if (ctx->d_mask.n < n) ctx->d_mask.alloc(n);
+        if (ctx->d_mask.n < n) ctx->d_mask.alloc(n, ctx->stream);
         CK(cudaMemcpyAsync(ctx->d_mask.p, mask, n, cudaMemcpyHostToDevice, ctx->stream));
         dm = ctx->d_mask.p;
     }
@@ -1545,7 +1527,7 @@ int32_t dmt_accept_counts(dmt_ctx *ctx, int32_t layout, uint32_t it0, uint32_t i
         Layout &L = layout_of(ctx, layout);
         REQUIRE(counts && it0 <= it1 && it1 < (uint32_t)L.dev.hist_len, DMT_ERR_ARG, "bad history range");
         DevBuf<unsigned long long> d;
-        d.alloc(L.nb);
+        d.alloc(L.nb, ctx->stream);
         ++g_launches, accept_counts_kernel<<<chain_grid(ctx, L.nb, 128), 128, 0, ctx->stream>>>(L.d_acc_hist.p, L.nb, ctx->M, it0, it1, d.p);
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(counts, d.p, sizeof(int64_t) * L.nb, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1562,7 +1544,7 @@ static void xfer_guiding(dmt_ctx *ctx, int side, int store, int k, double *H, do
     REQUIRE(H && F && c, DMT_ERR_ARG, "null");
     const size_t n = ctx->nsteps[k] + 1, P = ctx->P, D = ctx->D;
     DevBuf<double> dH, dF, dc;
-    dH.alloc(n * D * D * P, false); dF.alloc(n * D * P, false); dc.alloc(n * P, false);
+    dH.alloc_uninit(n * D * D * P); dF.alloc_uninit(n * D * P); dc.alloc_uninit(n * P);
     if (upload) {
         CK(cudaMemcpyAsync(dH.p, H, dH.n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
         CK(cudaMemcpyAsync(dF.p, F, dF.n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
@@ -1670,7 +1652,7 @@ int32_t dmt_debug_normals(dmt_ctx *ctx, uint32_t chain0, uint32_t tile0, uint32_
         REQUIRE(out && n_chains > 0 && n_tiles > 0, DMT_ERR_ARG, "bad arguments");
         const size_t n = (size_t)n_chains * n_tiles * 4 * ctx->DW;
         DevBuf<double> d;
-        d.alloc(n, false);
+        d.alloc_uninit(n);
         const int tot = n_chains * n_tiles;
         dim3 grid((tot + 127) / 128);
         switch (ctx->DW) {
@@ -1689,7 +1671,7 @@ int32_t dmt_debug_exponentials(dmt_ctx *ctx, uint32_t chain0, uint32_t iter, uin
         REQUIRE(out && n_chains > 0 && n_blocks > 0, DMT_ERR_ARG, "bad arguments");
         const int tot = n_chains * n_blocks;
         DevBuf<double> d;
-        d.alloc(tot, false);
+        d.alloc_uninit(tot);
         ++g_launches, debug_exponentials_kernel<<<(tot + 127) / 128, 128, 0, ctx->stream>>>(ctx->cfg.seed, chain0, iter, layout, n_chains, n_blocks, d.p);
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(out, d.p, tot * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1725,8 +1707,8 @@ int32_t dmt_p2p_export(dmt_ctx *ctx, uint8_t *handle64) {
         static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
         if (!ctx->p2p_local) {
             CK(cudaMalloc(&ctx->p2p_local, sizeof(P2PBuf)));
-            CK(cudaMemset(ctx->p2p_local, 0, sizeof(P2PBuf)));
-            CK(cudaDeviceSynchronize());
+            CK(cudaMemsetAsync(ctx->p2p_local, 0, sizeof(P2PBuf), ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
         }
         cudaIpcMemHandle_t h;
         CK(cudaIpcGetMemHandle(&h, ctx->p2p_local));
@@ -1804,9 +1786,9 @@ void pm_xfer(dmt_ctx *c, double *A, int n, const int32_t *chains, double *host, 
     const size_t len = (size_t)c->NP * c->D * n;
     DevBuf<double> nat;
     DevBuf<int> sel;
-    nat.alloc(len, false);
+    nat.alloc_uninit(len);
     if (chains) {
-        sel.alloc(n, false);
+        sel.alloc_uninit(n);
         CK(cudaMemcpyAsync(sel.p, chains, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
     }
     if (upload) CK(cudaMemcpyAsync(nat.p, host, len * sizeof(double), cudaMemcpyHostToDevice, c->stream));
@@ -1878,21 +1860,17 @@ int32_t dmt_get_pset_path_moments(dmt_ctx *ctx, double *mean, double *var, doubl
         REQUIRE(ctx->pm_count > 0, DMT_ERR_STATE, "no path moments accumulated (dmt_path_moments_add)");
         const int M = ctx->M, P = ctx->P;
         if (!ctx->d_pm_cs.p) { // chains of every pset in ascending order
-            std::vector<int> pset(M), cs(P + 1, 0), list(M);
-            CK(cudaMemcpy(pset.data(), ctx->d_pset.p, sizeof(int) * M, cudaMemcpyDeviceToHost));
-            for (int c = 0; c < M; c++) cs[pset[c] + 1]++;
+            std::vector<int> cs(P + 1, 0), list(M);
+            for (int c = 0; c < M; c++) cs[ctx->pset[c] + 1]++;
             for (int q = 0; q < P; q++) cs[q + 1] += cs[q];
             std::vector<int> fill(cs.begin(), cs.end() - 1);
-            for (int c = 0; c < M; c++) list[fill[pset[c]]++] = c;
-            ctx->d_pm_cs.alloc(P + 1, false);
-            ctx->d_pm_chains.alloc(M, false);
-            CK(cudaMemcpy(ctx->d_pm_cs.p, cs.data(), sizeof(int) * (P + 1), cudaMemcpyHostToDevice));
-            CK(cudaMemcpy(ctx->d_pm_chains.p, list.data(), sizeof(int) * M, cudaMemcpyHostToDevice));
-            CK(cudaStreamSynchronize(cudaStreamLegacy)); // pageable H2D copies return before the DMA lands; ctx->stream does not order against them
+            for (int c = 0; c < M; c++) list[fill[ctx->pset[c]]++] = c;
+            ctx->d_pm_cs.upload(cs, ctx->stream);
+            ctx->d_pm_chains.upload(list, ctx->stream);
         }
         const size_t len = (size_t)ctx->NP * ctx->D * P, t = pm_tile_len(ctx);
         DevBuf<double> out;
-        out.alloc(3 * len, false);
+        out.alloc_uninit(3 * len);
         int nk_max = 0;
         for (int k = 0; k < ctx->K; k++) nk_max = std::max(nk_max, ctx->nsteps[k] + 1);
         const size_t per_k = (size_t)nk_max * ctx->D * P;
